@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- frames/s of the splat render hot path (preprocess | sort | blend).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg3]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg3] [--dump-outputs DIR]
 
 A "step" is one frame: GaussianRenderer.prepare + render of one camera of the 36-view orbit
 (BASELINE.md section 3) over a synthetic cloud that is already resident in HBM (PointCloud::new is
@@ -18,6 +18,11 @@ BASELINE.json's metric and target are quoted on: 6M Gaussians, 1920x1080, SH deg
                        Rust+WGSL on wgpu/Vulkan and cannot run here) timed on one frame
 
 --impl reference runs that CPU oracle as the reference arm (oracle/_ref cannot be built).
+
+--dump-outputs DIR writes, after the timed steps, the frame of the last timed step (single-GPU arm or reference arm)
+as DIR/image.npy, float32 [H, W, 4].  A frame larger than DUMP_PIXELS pixels is written as a fixed, seeded sample
+of DUMP_PIXELS pixels, image.npy [DUMP_PIXELS, 4], with their row-major pixel indices in DIR/image_pixel_index.npy
+(float64).  The inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -37,17 +42,20 @@ METRIC = "frames/sec"
 REFERENCE_BUDGET_S = 120.0                  # host seconds the reference arm may spend on timed frames
 KERNELS_STAGE1 = 3                          # count, scan, preprocess
 KERNELS_BINNING = 3                         # count, scan, expand (per slab; the tile ranges are fused into the last onesweep pass)
+DUMP_PIXELS = 1 << 21                       # --dump-outputs: a 1920x1080 frame (33 MB as f32) is written whole, larger
+                                            # frames as this many sampled pixels (32 MB + 16 MB of indices)
+
+
+# the HBM bandwidth every roofline fraction is priced at: device-to-device copy bandwidth, median of 7 runs of 20 copies
+# of 4 GiB (torch copy_, CUDA events) on an NVIDIA B200 at a 1000 W power limit, 1965 MHz max SM clock.  Part of the
+# source so that every checkout prices alike (the round-1/2 numbers in DESIGN.md and profiles/ used 6570.9 GB/s, an
+# earlier per-machine measurement).
+HBM_PEAK_GBS = 6655.0
+SM_MAX_MHZ = 1965.0
 
 
 def measured_peaks():
-    p = os.path.join(ROOT, "MEASURED_PEAKS.json")
-    if os.path.exists(p):
-        try:
-            d = json.load(open(p))
-            return float(d["hbm_gbs"]), "measured (MEASURED_PEAKS.json)", float(d.get("sm_max_mhz", 1965.0))
-        except Exception:
-            pass
-    return 6650.0, "fallback (B200_PROFILING.md)", 1965.0
+    return HBM_PEAK_GBS, "measured D2D copy bandwidth, NVIDIA B200 at 1000 W (bench.py HBM_PEAK_GBS)", SM_MAX_MHZ
 
 
 class ClockSampler(threading.Thread):
@@ -114,6 +122,18 @@ def frame_crc(host):
     return "%08x" % (zlib.crc32(a.tobytes()) & 0xffffffff)
 
 
+def dump_outputs(path, image):
+    """--dump-outputs: the frame as float32 [H, W, 4], or a fixed seeded sample of DUMP_PIXELS of its pixels"""
+    img = np.asarray(image, dtype=np.float32)
+    H, W, C = img.shape
+    os.makedirs(path, exist_ok=True)
+    if H * W > DUMP_PIXELS:
+        idx = np.sort(np.random.default_rng(0).choice(H * W, size=DUMP_PIXELS, replace=False))
+        img = img.reshape(H * W, C)[idx]
+        np.save(os.path.join(path, "image_pixel_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(path, "image.npy"), img)
+
+
 CHECKSUM_VIEW = 0                           # index into the workload's camera list
 
 
@@ -127,9 +147,15 @@ def host_threads():
 
 
 def make_workload(name):
+    import hashlib
+    import tempfile
     import websplat_b200 as ws
     n, W, H, seed, compressed = ws.synth.CONFIGS[name]
-    cache = os.path.join("/tmp", "ws_cloud_%s.npz" % name)
+    # generating cfg3 takes ~15 s of host time, so the cloud is cached in the temporary directory; the file name carries a
+    # hash of the generator, so a cloud made by another version of synth.py is never picked up
+    with open(ws.synth.__file__, "rb") as f:
+        gen_hash = hashlib.sha1(f.read()).hexdigest()[:12]
+    cache = os.path.join(tempfile.gettempdir(), "ws_cloud_%s_%s.npz" % (name, gen_hash))
     cloud = None
     if os.path.exists(cache):
         try:
@@ -161,7 +187,7 @@ def frame_args(ws, cloud, view, W, H):
 
 
 def oracle_frame_seconds(cloud, view, W, H, repeats=1):
-    """One full frame of the CPU oracle (stage 1 -> stable u32 sort -> back-to-front composite)."""
+    """One full frame of the CPU oracle (stage 1 -> stable u32 sort -> back-to-front composite): (seconds, threads, image)."""
     import websplat_b200 as ws
     from oracle import oracle as orc
     orc.set_num_threads(host_threads())
@@ -169,10 +195,10 @@ def oracle_frame_seconds(cloud, view, W, H, repeats=1):
     best = None
     for _ in range(repeats):
         t0 = time.perf_counter()
-        orc.render_frame(cloud, view[0], view[1], W, H, fovx, fovy)
+        image = orc.render_frame(cloud, view[0], view[1], W, H, fovx, fovy)["image"]
         dt = time.perf_counter() - t0
         best = dt if best is None else min(best, dt)
-    return best, orc.num_threads()
+    return best, orc.num_threads(), image
 
 
 def run_reference(args):
@@ -201,8 +227,10 @@ def run_reference(args):
     args.steps = timed
     t0 = time.perf_counter()
     for i in range(args.steps):
-        oracle_frame_seconds(cloud, views[i % len(views)], W, H)
+        _, _, image = oracle_frame_seconds(cloud, views[i % len(views)], W, H)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, image)
     fps = args.steps / dt
     cores = orc.num_threads()
     line = {
@@ -303,6 +331,8 @@ def run_ours(args):
     ms_total = e0.elapsed_time(e1)
     clocks = sampler.finish()
     fps = K / (ms_total * 1e-3)
+    # the frame of the last timed step, taken before the e2e section below reuses the targets
+    last_frame = targets[(Wu + K - 1) % depth].cpu().numpy() if args.dump_outputs else None
 
     # ---- e2e: host buffers, uniforms H2D + frame D2H inside the timed region ----------------------
     # The public API is asynchronous on the caller's stream, so a caller that wants throughput keeps
@@ -476,7 +506,7 @@ def run_ours(args):
     # ---- CPU baseline: one frame of the same workload on the host cores -------------------------
     cpu = None
     if not args.no_cpu_baseline:
-        secs, cores = oracle_frame_seconds(cloud, views[0], W, H)
+        secs, cores, _ = oracle_frame_seconds(cloud, views[0], W, H)
         cpu = {"value": 1.0 / secs, "unit": "frames/s", "cores": cores, "kind": "port",
                "sample": "1 full frame (view 0) of the same workload on the CPU oracle: %.2f s" % secs}
 
@@ -502,6 +532,8 @@ def run_ours(args):
         "gpu_launches": K * (KERNELS_STAGE1 + depth_passes + (2 if split else 1) * (KERNELS_BINNING + tile_passes + 1)),
         "clocks": clocks,
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_frame)
     if rank == 0:
         print(json.dumps(line))
     return 0
@@ -521,7 +553,13 @@ def main():
                          "(the smaller the per-GPU share, the more latency-bound a single frame is)")
     ap.add_argument("--no-occlusion-split", action="store_true", help="single-GPU arm: bin / tile-sort / composite all pairs in one pass")
     ap.add_argument("--equal-bands", action="store_true", help="multi-GPU arm: keep the equal tile-row split instead of cost-balanced bands")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the frame of the last one as DIR/image.npy (float32; see the module docstring)")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.gpus > 1 and args.impl == "ours":
+        ap.error("--dump-outputs is implemented for the single-GPU and reference arms")
     if args.steps is None:
         args.steps = 360 if args.impl == "ours" else 10    # 10 orbits (~1 s of GPU time) / ~2-5 s per CPU frame
     if args.impl == "reference":

@@ -1,9 +1,12 @@
-"""The bench.py contract that can be checked without a GPU: the reference arm (CPU oracle) prints ONE JSON line with the
-keys the driver reads, and the GPU arm refuses to run without a CUDA device (no CPU fallback)."""
+"""The bench.py contract: the reference arm (CPU oracle) prints ONE JSON line with the keys a consumer of the result reads,
+the GPU arm refuses to run without a CUDA device (no CPU fallback), and --dump-outputs writes the frame of the last timed
+step (checked on the CPU through the reference arm, and on a GPU through the single-GPU arm)."""
 import json
 import os
 import subprocess
 import sys
+
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -68,3 +71,60 @@ def test_frame_crc_is_a_full_frame_hash():
         b = a.copy(); b[y, x, ch] = np.float16(6.1e-5)
         assert bench.frame_crc(b) != c0
     assert bench.frame_crc(a.copy()) == c0 and len(c0) == 8
+
+
+def test_reference_arm_dumps_the_frame_of_its_last_step(tmp_path):
+    """--dump-outputs: the image the timed path computed, as float32 (cfg1 has one view, so every step renders it)"""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    import websplat_b200 as ws
+    from oracle import oracle as orc
+    p = _run("--impl", "reference", "--workload", "cfg1", "--steps", "2", "--warmup", "0", "--dump-outputs", str(tmp_path))
+    assert p.returncode == 0, p.stderr[-2000:]
+    assert sorted(os.listdir(tmp_path)) == ["image.npy"]
+    img = np.load(tmp_path / "image.npy")
+    cloud, W, H, views = bench.make_workload("cfg1")
+    fovx, fovy = ws.synth.fov_for_viewport(W, H)
+    want = orc.render_frame(cloud, views[0][0], views[0][1], W, H, fovx, fovy)["image"]
+    assert img.dtype == np.float32 and np.array_equal(img, want)
+
+
+def test_dump_outputs_samples_a_large_frame(tmp_path):
+    """a frame above DUMP_PIXELS pixels is written as a fixed seeded pixel sample plus its indices, within 64 MB"""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    H, W = 2160, 3840
+    frame = np.random.default_rng(3).random((H, W, 4)).astype(np.float16)
+    bench.dump_outputs(str(tmp_path / "a"), frame)
+    bench.dump_outputs(str(tmp_path / "b"), frame[::-1].copy())
+    img, idx = np.load(tmp_path / "a" / "image.npy"), np.load(tmp_path / "a" / "image_pixel_index.npy")
+    assert img.dtype == np.float32 and idx.dtype == np.float64 and img.shape == (bench.DUMP_PIXELS, 4) and idx.shape == (bench.DUMP_PIXELS,)
+    assert np.array_equal(img, frame.reshape(-1, 4)[idx.astype(np.int64)].astype(np.float32))
+    assert np.array_equal(idx, np.load(tmp_path / "b" / "image_pixel_index.npy"))      # the sample does not depend on the frame
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= 64e6
+
+
+@pytest.mark.gpu
+def test_gpu_arm_dumps_the_frame_of_its_last_step(ctx, tmp_path):
+    """--dump-outputs of the single-GPU arm: the RGBA16F frame of the last timed step, as float32, equal to the same view
+    rendered through the API (cfg1 has one view, so every step renders it)"""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    import websplat_b200 as ws
+    p = _run("--workload", "cfg1", "--steps", "5", "--warmup", "2", "--no-cpu-baseline", "--no-extra", "--dump-outputs", str(tmp_path))
+    assert p.returncode == 0, p.stderr[-2000:]
+    assert json.loads(p.stdout.strip().splitlines()[-1])["steps"] == 5
+    img = np.load(tmp_path / "image.npy")
+    cloud, W, H, views = bench.make_workload("cfg1")
+    pc = ws.PointCloud.new(ctx, ws.GenericGaussianPointCloud(cloud["gaussians"], cloud["sh_coefs"], cloud["sh_deg"], cloud["num_points"],
+                                                              ws.Aabb(cloud["aabb_min"], cloud["aabb_max"]), cloud["center"]))
+    r = ws.GaussianRenderer.new(ctx, ws.FORMAT_RGBA16_FLOAT, cloud["sh_deg"], False)
+    r.prepare(None, pc, bench.frame_args(ws, cloud, views[0], W, H))
+    target = torch.empty((H, W, 4), dtype=torch.float16, device="cuda")
+    r.render(target, pc)
+    torch.cuda.synchronize()
+    assert img.dtype == np.float32 and np.array_equal(img, target.cpu().numpy().astype(np.float32))
