@@ -4,6 +4,7 @@ use std::os::raw::{c_char, c_int, c_void};
 
 pub const WS_OK: i32 = 0;
 pub const WS_ERR_PAIR_OVERFLOW: i32 = -4;
+pub const WS_MAX_VIEWS: usize = 8;
 
 #[repr(C)] #[derive(Copy, Clone, Default, Debug)] pub struct ws_aabb { pub min: [f32; 3], pub max: [f32; 3] }
 #[repr(C)] #[derive(Copy, Clone, Default)] pub struct ws_quantization { pub zero_point: i32, pub scale: f32, pub _pad: [u32; 2] }
@@ -74,6 +75,10 @@ extern "C" {
     pub fn ws_renderer_render(r: *mut ws_renderer, pc: *mut ws_pointcloud, dst_device: *mut c_void, row_pitch: usize, clear: *const f64, stream: *mut c_void) -> i32;
     pub fn ws_renderer_render_to_host(r: *mut ws_renderer, pc: *mut ws_pointcloud, dst_host: *mut c_void, row_pitch: usize, clear: *const f64, stream: *mut c_void) -> i32;
     pub fn ws_renderer_num_visible_points(r: *mut ws_renderer, out: *mut u32) -> i32;
+    pub fn ws_renderer_prepare_views(r: *mut ws_renderer, pc: *mut ws_pointcloud, args: *const ws_splatting_args, num_views: u32, stream: *mut c_void) -> i32;
+    pub fn ws_renderer_render_views(r: *mut ws_renderer, pc: *mut ws_pointcloud, dst_device: *mut c_void, row_pitch: usize, view_stride: usize, clear: *const f64, stream: *mut c_void) -> i32;
+    pub fn ws_renderer_render_views_to_host(r: *mut ws_renderer, pc: *mut ws_pointcloud, dst_host: *mut c_void, row_pitch: usize, view_stride: usize, clear: *const f64, stream: *mut c_void) -> i32;
+    pub fn ws_renderer_views_num_visible_points(r: *mut ws_renderer, out: *mut u32, count: u32) -> i32;
     pub fn ws_renderer_stats(r: *mut ws_renderer, out: *mut ws_frame_stats) -> i32;
     pub fn ws_renderer_set_pair_capacity(r: *mut ws_renderer, max_pairs: u64) -> i32;
 }

@@ -144,13 +144,13 @@ pub enum ColorFormat { Rgba8Unorm = 0, Rgba16Float = 1, Rgba32Float = 2 }
 impl ColorFormat { pub fn bytes_per_pixel(self) -> usize { match self { Self::Rgba8Unorm => 4, Self::Rgba16Float => 8, Self::Rgba32Float => 16 } } }
 
 /// `GaussianRenderer` (src/renderer.rs:20-31).  Not re-entrant, like `&mut self` upstream.
-pub struct GaussianRenderer { h: *mut ffi::ws_renderer, format: ColorFormat }
+pub struct GaussianRenderer { h: *mut ffi::ws_renderer, format: ColorFormat, views: u32 }
 impl GaussianRenderer {
     /// `GaussianRenderer::new` (src/renderer.rs:33).
     pub fn new(ctx: &Context, color_format: ColorFormat, sh_deg: u32, compressed: bool) -> Result<Self> {
         let mut h = std::ptr::null_mut();
         check(unsafe { ffi::ws_renderer_create(ctx.h, color_format as i32, sh_deg, compressed as i32, &mut h) })?;
-        Ok(Self { h, format: color_format })
+        Ok(Self { h, format: color_format, views: 0 })
     }
     /// `prepare` (src/renderer.rs:191): enqueues stage 1 + 2 on `stream`.
     ///
@@ -178,6 +178,38 @@ impl GaussianRenderer {
     pub fn num_visible_points(&self) -> Result<u32> {
         let mut v = 0u32;
         check(unsafe { ffi::ws_renderer_num_visible_points(self.h, &mut v) })?;
+        Ok(v)
+    }
+    /// A batch of up to `ffi::WS_MAX_VIEWS` views of one cloud (one viewport): stage 1 + 2 for all of them. Every view
+    /// renders bit-identical to the same view through `prepare` + `render`.
+    pub fn prepare_views(&mut self, stream: Stream, pc: &PointCloud, render_settings: &[SplattingArgs]) -> Result<()> {
+        let a: Vec<ffi::ws_splatting_args> = render_settings.iter().map(ffi::ws_splatting_args::from).collect();
+        check(unsafe { ffi::ws_renderer_prepare_views(self.h, pc.h, a.as_ptr(), a.len() as u32, stream.0) })?;
+        self.views = a.len() as u32;
+        Ok(())
+    }
+    /// Stage 3 of the batch into device memory: view v starts at `target_device + v * view_stride`.
+    ///
+    /// # Safety
+    /// `target_device` must point at `views * view_stride` bytes of device memory of the renderer's colour format.
+    pub unsafe fn render_views(&self, stream: Stream, pc: &PointCloud, target_device: *mut c_void, row_pitch: usize, view_stride: usize,
+                               clear: [f64; 4]) -> Result<()> {
+        check(ffi::ws_renderer_render_views(self.h, pc.h, target_device, row_pitch, view_stride, clear.as_ptr(), stream.0))
+    }
+    /// The batch into `target_host`, tightly packed: view v at byte `v * width * height * bytes_per_pixel`
+    /// (asynchronously on `stream`).
+    pub fn render_views_to_host(&self, stream: Stream, pc: &PointCloud, target_host: &mut [u8], width: u32, height: u32, clear: [f64; 4]) -> Result<()> {
+        let pitch = width as usize * self.format.bytes_per_pixel();
+        let stride = pitch * height as usize;
+        if target_host.len() < stride * self.views as usize {
+            return Err(anyhow!("websplat_b200: host buffer smaller than the batch"));
+        }
+        check(unsafe { ffi::ws_renderer_render_views_to_host(self.h, pc.h, target_host.as_mut_ptr() as *mut c_void, pitch, stride, clear.as_ptr(), stream.0) })
+    }
+    /// Per-view visible point counts of the last batch (blocking).
+    pub fn views_num_visible_points(&self) -> Result<Vec<u32>> {
+        let mut v = vec![0u32; self.views as usize];
+        check(unsafe { ffi::ws_renderer_views_num_visible_points(self.h, v.as_mut_ptr(), self.views) })?;
         Ok(v)
     }
     /// The `GPUStopwatch` replacement: "preprocess" / "sorting" / "rasterization" (src/renderer.rs:220-239) as ms.

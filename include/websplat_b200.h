@@ -271,6 +271,37 @@ WS_API ws_status ws_renderer_set_cuda_graphs(ws_renderer *r, int32_t enabled);
  * in the WS_BUF_PAIR_* / WS_BUF_TILE_RANGES read-backs (with the split they describe the far slab). */
 WS_API ws_status ws_renderer_set_occlusion_split(ws_renderer *r, int32_t enabled);
 
+/* ---- batches of views (new: the reference renders one view per prepare / render) --------------
+ * K <= WS_MAX_VIEWS cameras of ONE cloud in one frame: stage 1 reads the cloud once for all views, stages 2-3 run
+ * once over the K views stacked into one frame of K x tiles rows.  Every view is bit-identical to the same view
+ * rendered alone through ws_renderer_prepare + ws_renderer_render.
+ *  - args[0..num_views) must share the viewport; everything else (camera, clipping box, max_sh_deg, mip splatting,
+ *    kernel size, gaussian_scaling, walltime) may differ.  Each view is checked like a single frame; in addition
+ *    num_views of 0 or above WS_MAX_VIEWS, different viewports, a sharded renderer, render / render_to_host after
+ *    prepare_views and render_views after prepare fail with WS_ERR_INVALID_ARGUMENT, and num_views x num_points
+ *    >= 2^30 with WS_ERR_UNSUPPORTED.
+ *  - after a batch, ws_renderer_read_buffer, ws_renderer_camera_uniform and ws_renderer_settings_uniform return
+ *    WS_ERR_UNSUPPORTED.  ws_renderer_stats reports num_visible = sum of the per-view counts, num_pairs = the pairs of
+ *    the batch, num_tiles = K x tiles, width / height of one view and the stage times of the whole batch;
+ *    ws_renderer_num_visible_points returns the sum as well.
+ *  - deferred frame status, the automatic pair capacity (K x max(8 N, 1<<22): what the views get one by one) and CUDA graphs (a graph of its own, so
+ *    alternating single frames and batches does not recapture) work as for one frame.  The sort buffers are sized for
+ *    K x N points: a renderer that alternates single frames and batches reallocates them at every switch; use one
+ *    renderer per mode to avoid that. */
+#define WS_MAX_VIEWS 8
+/* stage 1 + 2 for num_views cameras of one cloud. Asynchronous. */
+WS_API ws_status ws_renderer_prepare_views(ws_renderer *r, ws_pointcloud *pc, const ws_splatting_args *args,
+                                           uint32_t num_views, void *cuda_stream);
+/* stage 3 of the batch: view v lands at dst + v * view_stride_bytes (view_stride_bytes >= height * row_pitch_bytes,
+ * a multiple of the pixel size). Asynchronous. */
+WS_API ws_status ws_renderer_render_views(ws_renderer *r, ws_pointcloud *pc, void *dst_rgba_device, size_t row_pitch_bytes,
+                                          size_t view_stride_bytes, const double clear[4], void *cuda_stream);
+/* the same into an internal device buffer, then async copies to host memory (layout as above) */
+WS_API ws_status ws_renderer_render_views_to_host(ws_renderer *r, ws_pointcloud *pc, void *dst_rgba_host, size_t row_pitch_bytes,
+                                                  size_t view_stride_bytes, const double clear[4], void *cuda_stream);
+/* per-view visible point counts V_v of the last batch into out[0..num_views) (count >= num_views). Synchronises. */
+WS_API ws_status ws_renderer_views_num_visible_points(ws_renderer *r, uint32_t *out, uint32_t count);
+
 /* ---- intermediate read-back (parity tests; synchronises) -------------------
  * Copies an intermediate buffer of the LAST prepared frame to host memory. */
 typedef enum {

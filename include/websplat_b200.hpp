@@ -178,8 +178,8 @@ public:
         return r;
     }
     ~GaussianRenderer() { ws_renderer_destroy(h_); }
-    GaussianRenderer(GaussianRenderer &&o) noexcept : h_(o.h_) { o.h_ = nullptr; }
-    GaussianRenderer &operator=(GaussianRenderer &&o) noexcept { std::swap(h_, o.h_); return *this; }
+    GaussianRenderer(GaussianRenderer &&o) noexcept : h_(o.h_), views_(o.views_) { o.h_ = nullptr; }
+    GaussianRenderer &operator=(GaussianRenderer &&o) noexcept { std::swap(h_, o.h_); std::swap(views_, o.views_); return *this; }
     GaussianRenderer(const GaussianRenderer &) = delete;
     GaussianRenderer &operator=(const GaussianRenderer &) = delete;
 
@@ -204,6 +204,34 @@ public:
     }
     /// num_visible_points (renderer.rs:170): blocking read-back of V
     uint32_t num_visible_points() { uint32_t v = 0; check(ws_renderer_num_visible_points(h_, &v)); return v; }
+    /// batch of up to WS_MAX_VIEWS views of one cloud (one viewport): stage 1 + 2 for all of them
+    void prepare_views(void *stream, const PointCloud &pc, const std::vector<SplattingArgs> &render_settings)
+    {
+        std::vector<ws_splatting_args> a;
+        a.reserve(render_settings.size());
+        for (const SplattingArgs &s : render_settings) a.push_back(s.c());
+        check(ws_renderer_prepare_views(h_, pc.handle(), a.data(), (uint32_t)a.size(), stream));
+        views_ = (uint32_t)a.size();
+    }
+    /// stage 3 of the batch into DEVICE memory: view v at target_device + v * view_stride
+    void render_views(void *stream, const PointCloud &pc, void *target_device, size_t row_pitch, size_t view_stride,
+                      const std::array<double, 4> &clear)
+    {
+        check(ws_renderer_render_views(h_, pc.handle(), target_device, row_pitch, view_stride, clear.data(), stream));
+    }
+    /// the same into host memory (asynchronously on `stream`)
+    void render_views_to_host(void *stream, const PointCloud &pc, void *target_host, size_t row_pitch, size_t view_stride,
+                              const std::array<double, 4> &clear)
+    {
+        check(ws_renderer_render_views_to_host(h_, pc.handle(), target_host, row_pitch, view_stride, clear.data(), stream));
+    }
+    /// per-view visible point counts of the last batch (blocking)
+    std::vector<uint32_t> views_num_visible_points()
+    {
+        std::vector<uint32_t> v(views_);
+        check(ws_renderer_views_num_visible_points(h_, v.data(), views_));
+        return v;
+    }
     /// the GPUStopwatch replacement: "preprocess" / "sorting" / "rasterization" (renderer.rs:220-239) in ms; synchronises
     ws_frame_stats stats() { ws_frame_stats s; check(ws_renderer_stats(h_, &s)); return s; }
     ws_format color_format() const { return ws_renderer_color_format(h_); }
@@ -214,6 +242,7 @@ public:
 private:
     GaussianRenderer() = default;
     ws_renderer *h_ = nullptr;
+    uint32_t views_ = 0;       // views of the last prepare_views
 };
 
 // ---- dataset cameras (src/scene.rs) -----------------------------------------------------------------------------

@@ -1,4 +1,4 @@
-"""Offline dataset renderer: `python scripts/render_scene.py <input.ply|.npz> <cameras.json> <img_out> [--max-sh-deg N]`.
+"""Offline dataset renderer: `python scripts/render_scene.py <input.ply|.npz> <cameras.json> <img_out> [--max-sh-deg N] [--batch K]`.
 The B200 counterpart of the reference's `render` binary (bin/render.rs:14-180): renders the test split, then the
 train split, of a 3DGS cameras.json to PNG files."""
 import argparse
@@ -14,7 +14,11 @@ def main():
     ap = argparse.ArgumentParser(description="Dataset offline renderer. Renders to PNG files")
     ap.add_argument("input"); ap.add_argument("scene"); ap.add_argument("img_out")
     ap.add_argument("--max-sh-deg", type=int, default=3)
+    ap.add_argument("--batch", type=int, default=1,
+                    help="render up to this many consecutive cameras of equal resolution together (1..%d)" % ws.MAX_VIEWS)
     opt = ap.parse_args()
+    if not 1 <= opt.batch <= ws.MAX_VIEWS:
+        ap.error("--batch must be in [1, %d]" % ws.MAX_VIEWS)
     print("reading scene file '%s'" % opt.scene)
     scene = ws.Scene.from_json(opt.scene)
     ctx = ws.Context(0)
@@ -24,7 +28,7 @@ def main():
     for split in (ws.scene.TEST, ws.scene.TRAIN):
         cams = scene.cameras(split)
         t0 = time.perf_counter()
-        ws.scene.render_views(ws, ctx, renderer, pc, cams, opt.img_out, split)
+        ws.scene.render_views(ws, ctx, renderer, pc, cams, opt.img_out, split, batch=opt.batch)
         print("rendering %s: %d views in %.2f s -> '%s'" % (split, len(cams), time.perf_counter() - t0, os.path.join(opt.img_out, split)))
     print("done!")
 

@@ -15,6 +15,7 @@ C ABI is mirrored here with the SAME names, argument meaning and error behaviour
     GaussianRenderer::new          renderer.rs:33      GaussianRenderer.new(ctx, fmt, sh_deg, compressed)
     GaussianRenderer::prepare      renderer.rs:191     GaussianRenderer.prepare(stream, pc, args)
     GaussianRenderer::render       renderer.rs:250     GaussianRenderer.render(target, pc, clear, stream)
+    (new: K views of one cloud)                        GaussianRenderer.prepare_views / render_views
     num_visible_points             renderer.rs:170     GaussianRenderer.num_visible_points()
     GPUStopwatch                   utils.rs:26-134     GaussianRenderer.stats()
 
@@ -144,7 +145,10 @@ EXPORTED_SYMBOLS = [
     "ws_renderer_shard_exchange", "ws_renderer_shard_finish", "ws_renderer_shard_band", "ws_renderer_render_band",
     "ws_renderer_render_band_to_root", "ws_renderer_shard_frame", "ws_renderer_shard_download",
     "ws_renderer_shard_frame_to_root", "ws_renderer_shard_set_bands", "ws_renderer_shard_get_bands", "ws_renderer_shard_set_gated",
+    "ws_renderer_prepare_views", "ws_renderer_render_views", "ws_renderer_render_views_to_host", "ws_renderer_views_num_visible_points",
 ]
+
+MAX_VIEWS = 8              # WS_MAX_VIEWS: views per batch
 
 _lib = None
 
@@ -226,6 +230,10 @@ def lib():
         "ws_renderer_shard_get_bands": (i32, [vp, C.POINTER(u32), u32]),
         "ws_renderer_shard_set_gated": (i32, [vp, i32]),
         "ws_renderer_shard_frame_to_root": (i32, [vp, vp, C.POINTER(ws_splatting_args), u32, C.POINTER(C.c_double * 4), vp]),
+        "ws_renderer_prepare_views": (i32, [vp, vp, C.POINTER(ws_splatting_args), u32, vp]),
+        "ws_renderer_render_views": (i32, [vp, vp, vp, C.c_size_t, C.c_size_t, C.POINTER(C.c_double * 4), vp]),
+        "ws_renderer_render_views_to_host": (i32, [vp, vp, vp, C.c_size_t, C.c_size_t, C.POINTER(C.c_double * 4), vp]),
+        "ws_renderer_views_num_visible_points": (i32, [vp, C.POINTER(u32), u32]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)
@@ -648,6 +656,42 @@ class GaussianRenderer:
         row_pitch = self._viewport[0] * _BPP[self._format]
         clr = (C.c_double * 4)(*[float(c) for c in clear])
         _check(lib().ws_renderer_render_to_host(self._h, pc._h, C.c_void_p(ptr), row_pitch, C.byref(clr), _stream_handle(stream)))
+
+    def prepare_views(self, stream, pc, render_settings):
+        """Enqueue stage 1 + 2 for a batch of up to MAX_VIEWS views of `pc` (a list of SplattingArgs with one viewport).
+        Every view renders bit-identical to the same view through prepare + render."""
+        args = list(render_settings)
+        arr = (ws_splatting_args * max(len(args), 1))(*[a._c() for a in args])
+        self._viewport = args[0].viewport if args else self._viewport
+        self._views = len(args)
+        _check(lib().ws_renderer_prepare_views(self._h, pc._h, arr, len(args), _stream_handle(stream)))
+
+    def render_views(self, target, pc, clear=(0.0, 0.0, 0.0, 0.0), stream=None, row_pitch=None, view_stride=None):
+        """Enqueue stage 3 of the batch into `target`: a device pointer (int) or a CUDA torch tensor of K x H x W x 4
+        in the renderer's format; view v starts `view_stride` bytes after view v - 1 (default: H * row_pitch)."""
+        ptr = target if isinstance(target, int) else target.data_ptr()
+        if row_pitch is None:
+            row_pitch = self._viewport[0] * _BPP[self._format]
+        if view_stride is None:
+            view_stride = self._viewport[1] * row_pitch
+        clr = (C.c_double * 4)(*[float(c) for c in clear])
+        _check(lib().ws_renderer_render_views(self._h, pc._h, C.c_void_p(ptr), row_pitch, view_stride, C.byref(clr), _stream_handle(stream)))
+
+    def render_views_to_host(self, host_target, pc, clear=(0.0, 0.0, 0.0, 0.0), stream=None):
+        """render_views into host memory: a numpy array or a (pinned) CPU torch tensor of K x H x W x 4.  Asynchronous
+        on `stream`; synchronise before reading."""
+        ptr = host_target.ctypes.data if isinstance(host_target, np.ndarray) else host_target.data_ptr()
+        row_pitch = self._viewport[0] * _BPP[self._format]
+        clr = (C.c_double * 4)(*[float(c) for c in clear])
+        _check(lib().ws_renderer_render_views_to_host(self._h, pc._h, C.c_void_p(ptr), row_pitch, self._viewport[1] * row_pitch,
+                                                      C.byref(clr), _stream_handle(stream)))
+
+    def views_num_visible_points(self):
+        """Per-view visible point counts of the last batch (synchronises)."""
+        k = getattr(self, "_views", 0)
+        o = (C.c_uint32 * max(k, 1))()
+        _check(lib().ws_renderer_views_num_visible_points(self._h, o, k))
+        return [int(x) for x in o[:k]]
 
     def empty_host_frame(self):
         dt, ch = _NP_PIXEL[self._format]

@@ -763,7 +763,18 @@ struct ws_renderer {
     int flag_next = 0;
     uint64_t buf_generation = 0;           // bumped whenever a buffer a captured graph points into is (re)allocated
     struct { const ws_pointcloud *pc; uint64_t pc_gen, buf_gen; const void *gaussians, *scratch, *state; uint32_t n, W, H, pair_cap, n_cap; bool split; } prep_key = {};
+    // batch of views (ws_renderer_prepare_views): d_uniforms holds 1 + WS_MAX_VIEWS blocks, [0] = the "tall" frame of
+    // K * tiles_y tile rows that stages 2-3 see, [1 + v] = view v's own block for stage 1
+    uint32_t views = 1;                    // views of the prepared frame
+    bool batch = false;                    // the prepared frame is a batch (prepare_views)
+    uint32_t *d_view_visible = nullptr;    // WS_MAX_VIEWS per-view survivor counts (in d_scratch)
+    uint32_t *d_part_union = nullptr;      // per 256-Gaussian partition: survivors in any view (in d_scratch)
+    int grid_pre_views = 0;
+    FrameUniforms h_views[1 + WS_MAX_VIEWS];
+    cudaGraphExec_t views_exec = nullptr;  // its own graph, so alternating single frames and batches never recaptures
+    struct { const ws_pointcloud *pc; uint64_t pc_gen, buf_gen; const void *gaussians, *scratch, *state; uint32_t n, K, W, H, pair_cap, n_cap; bool split; } views_key = {};
 };
+static_assert(WS_MAX_VIEWS == MAX_VIEWS, "views per batch");
 
 static void free_shard(ws_renderer *r);
 static void free_sort_stuff(ws_renderer *r)
@@ -792,6 +803,7 @@ extern "C" void ws_renderer_destroy(ws_renderer *r)
     for (int i = 0; i < ws_renderer::FLAG_SLOTS; i++) if (r->ev_flags[i]) cudaEventDestroy(r->ev_flags[i]);
     if (r->h_flags) cudaFreeHost(r->h_flags);
     if (r->prep_exec) cudaGraphExecDestroy(r->prep_exec);
+    if (r->views_exec) cudaGraphExecDestroy(r->views_exec);
     if (r->cap_stream) cudaStreamDestroy(r->cap_stream);
     delete r;
 }
@@ -806,7 +818,7 @@ extern "C" ws_status ws_renderer_create(ws_context *ctx, ws_format fmt, uint32_t
     ws_renderer *r = new (std::nothrow) ws_renderer();
     if (!r) return fail(WS_ERR_OUT_OF_MEMORY, "host allocation failed");
     r->ctx = ctx; r->format = fmt; r->sh_deg = sh_deg; r->compressed = compressed != 0;
-    cudaError_t e = cudaMalloc(&r->d_uniforms, sizeof(FrameUniforms));
+    cudaError_t e = cudaMalloc(&r->d_uniforms, (1 + WS_MAX_VIEWS) * sizeof(FrameUniforms));
     if (e != cudaSuccess) { ws_status s = fail_cuda(e, "cudaMalloc uniforms"); ws_renderer_destroy(r); return s; }
     for (int i = 0; i < EV_COUNT; i++) {
         e = cudaEventCreate(&r->ev[i]);
@@ -820,6 +832,7 @@ extern "C" ws_status ws_renderer_create(ws_context *ctx, ws_format fmt, uint32_t
     r->grid_pre = ctx->sm_count * preprocess_blocks_per_sm(r->compressed);
     r->grid_sort = ctx->sm_count * sort_pass_blocks_per_sm();
     r->grid_bin = ctx->sm_count * binning_blocks_per_sm();
+    r->grid_pre_views = ctx->sm_count * preprocess_views_blocks_per_sm(r->compressed);
     {   // A/B knobs (profiles/): fewer resident CTAs per SM for the persistent kernels leave room for the other frame's kernels
         auto per_sm = [&](const char *name, int cur) { const char *e = getenv(name); const int k = e ? atoi(e) : 0; return (k >= 1 && k * ctx->sm_count < cur) ? k * ctx->sm_count : cur; };
         r->grid_pre = per_sm("WS_PRE_CTAS_PER_SM", r->grid_pre);
@@ -880,13 +893,14 @@ static int active_cull_default()
     return v;
 }
 
-// GPURSSorter::create_sort_stuff analogue (gpu_rs.rs:141-175, renderer.rs:200-211)
-static ws_status ensure_capacity(ws_renderer *r, uint32_t n, uint32_t tiles)
+// GPURSSorter::create_sort_stuff analogue (gpu_rs.rs:141-175, renderer.rs:200-211).  A batch of `views` views passes
+// n = views x N: its automatic pair capacity, views x max(8 N, 1<<22), is what its views would get one by one.
+static ws_status ensure_capacity(ws_renderer *r, uint32_t n, uint32_t tiles, uint32_t views = 1)
 {
     uint64_t want_pairs = r->pair_cap_req;
     if (want_pairs == 0) {
         want_pairs = (uint64_t)n * 8u;
-        if (want_pairs < (1u << 22)) want_pairs = 1u << 22;
+        if (want_pairs < (1ull << 22) * views) want_pairs = (1ull << 22) * views;
         if (want_pairs >= (1ull << 30)) want_pairs = (1ull << 30) - 1;
     }
     const uint32_t pair_cap = (uint32_t)want_pairs;
@@ -894,7 +908,8 @@ static ws_status ensure_capacity(ws_renderer *r, uint32_t n, uint32_t tiles)
         if (r->shard.world > 0 && r->d_scratch) return fail(WS_ERR_INVALID_ARGUMENT, "sharded renderer: capacities are fixed by ws_renderer_shard_configure");
         free_sort_stuff(r);
         const size_t nn = n ? n : 1;
-        const size_t parts256 = (nn + 255) / 256;
+        // + WS_MAX_VIEWS: a batch of K views of N points keeps K x ceil(N/256) partition counts, and n = K * N here
+        const size_t parts256 = (nn + 255) / 256 + WS_MAX_VIEWS;
         const size_t sparts_n = (nn + SORT_PART - 1) / SORT_PART;
         const size_t sparts_p = ((size_t)pair_cap + SORT_PART - 1) / SORT_PART;
         size_t off = 0;
@@ -905,6 +920,8 @@ static ws_status ensure_capacity(ws_renderer *r, uint32_t n, uint32_t tiles)
         const size_t o_sb = off; off = align_up(off + parts256 * 4, 256);
         const size_t o_pb = off; off = align_up(off + parts256 * 4, 256);
         const size_t o_bb = off; off = align_up(off + parts256 * 4, 256);
+        const size_t o_un = off; off = align_up(off + parts256 * 4, 256);
+        const size_t o_vv = off; off = align_up(off + WS_MAX_VIEWS * 4, 256);
         const size_t o_sd = off; off = align_up(off + 4 * sparts_n * 256 * 4, 256);
         const size_t o_st = off; off = align_up(off + 2 * 3 * sparts_p * 256 * 4, 256);     // x2: one set per depth slab
         const size_t gparts_n = (sparts_n + SORT_LB_GROUP - 1) / SORT_LB_GROUP, gparts_p = (sparts_p + SORT_LB_GROUP - 1) / SORT_LB_GROUP;
@@ -919,6 +936,8 @@ static ws_status ensure_capacity(ws_renderer *r, uint32_t n, uint32_t tiles)
         r->d_scan_bin = reinterpret_cast<uint32_t *>(r->d_scratch + o_sb);
         r->d_part_bases = reinterpret_cast<uint32_t *>(r->d_scratch + o_pb);
         r->d_bin_bases = reinterpret_cast<uint32_t *>(r->d_scratch + o_bb);
+        r->d_part_union = reinterpret_cast<uint32_t *>(r->d_scratch + o_un);
+        r->d_view_visible = reinterpret_cast<uint32_t *>(r->d_scratch + o_vv);
         r->d_status_depth = reinterpret_cast<uint32_t *>(r->d_scratch + o_sd);
         r->d_status_tile = reinterpret_cast<uint32_t *>(r->d_scratch + o_st);
         r->d_gstatus_depth = reinterpret_cast<uint32_t *>(r->d_scratch + o_gd);
@@ -997,11 +1016,11 @@ static ws_status validate_frame(ws_renderer *r, ws_pointcloud *pc, const ws_spla
 // depth-sorts (the whole cloud; total / world for sharded frames).  Automatic threshold: measured on one GPU cfg1
 // (100 K points) -14 %, cfg2 (1 M) -2 %, cfg3 (6 M) +7 % -- the six extra launches and the state round trip pay off only
 // when there are many pairs to save.
-static ws_status decide_split(ws_renderer *r, uint64_t points_here, uint32_t W, uint32_t H)
+static ws_status decide_split(ws_renderer *r, uint64_t points_here, uint32_t W, uint32_t H, uint32_t views = 1)
 {
     r->frame_split = r->split_mode == 1 || (r->split_mode == 2 && points_here >= 2000000u);
     if (r->frame_split) {
-        const size_t px = (size_t)W * H;
+        const size_t px = (size_t)W * H * views;
         if (r->state_px < px) {
             cudaFree(r->d_state); r->d_state = nullptr; r->state_px = 0;
             CU(cudaMalloc(&r->d_state, px * sizeof(float4)));
@@ -1012,6 +1031,8 @@ static ws_status decide_split(ws_renderer *r, uint64_t points_here, uint32_t W, 
     return WS_OK;
 }
 
+static void build_frame_uniforms(ws_renderer *r, ws_pointcloud *pc, const ws_splatting_args *args, FrameUniforms *out);
+
 // uniforms + per-frame clears (everything before stage 1)
 static ws_status begin_frame(ws_renderer *r, ws_pointcloud *pc, const ws_splatting_args *args, uint32_t capacity_points, cudaStream_t stream,
                             bool with_clears = true)
@@ -1019,11 +1040,28 @@ static ws_status begin_frame(ws_renderer *r, ws_pointcloud *pc, const ws_splatti
     const uint32_t W = args->viewport[0], H = args->viewport[1];
     const uint32_t tx = (W + TILE - 1) / TILE, ty = (H + TILE - 1) / TILE;
     const uint32_t tiles = tx * ty;
-    r->prepared = false; r->rendered = false;
+    r->prepared = false; r->rendered = false; r->batch = false; r->views = 1;
     ws_status st = ensure_capacity(r, capacity_points, tiles);
     if (st != WS_OK) return st;
 
     FrameUniforms &U = r->h_uniforms;
+    build_frame_uniforms(r, pc, args, &U);
+    r->tile_passes = (tiles > 65536u) ? 3 : ((tiles > 256u) ? 2 : 1);
+
+    // pageable source: the runtime stages the 0.5 KB before returning, so h_uniforms may be reused
+    CU(cudaMemcpyAsync(r->d_uniforms, &U, sizeof U, cudaMemcpyHostToDevice, stream));
+    if (with_clears) {
+        CU(cudaMemsetAsync(r->d_scratch, 0, r->scratch_bytes, stream));
+        CU(cudaMemsetAsync(r->d_ranges, 0xff, (size_t)r->tiles_cap * 8 * (r->frame_split ? 2 : 1), stream));    // {begin, ~end} identities for atomicMin (one set per depth slab)
+    }
+    return WS_OK;
+}
+
+static void build_frame_uniforms(ws_renderer *r, ws_pointcloud *pc, const ws_splatting_args *args, FrameUniforms *out)
+{
+    const uint32_t W = args->viewport[0], H = args->viewport[1];
+    const uint32_t tx = (W + TILE - 1) / TILE, ty = (H + TILE - 1) / TILE;
+    FrameUniforms &U = *out;
     build_camera_uniform(args, &U.cam);
     build_settings_uniform(args, pc, &U.rs);
     U.quant = pc->quant;
@@ -1037,15 +1075,6 @@ static ws_status begin_frame(ws_renderer *r, ws_pointcloud *pc, const ws_splatti
         U.inv_scene_extend = one / U.rs.scene_extend;
         U._padf[0] = U._padf[1] = U._padf[2] = 0.f;
     }
-    r->tile_passes = (tiles > 65536u) ? 3 : ((tiles > 256u) ? 2 : 1);
-
-    // pageable source: the runtime stages the 0.5 KB before returning, so h_uniforms may be reused
-    CU(cudaMemcpyAsync(r->d_uniforms, &U, sizeof U, cudaMemcpyHostToDevice, stream));
-    if (with_clears) {
-        CU(cudaMemsetAsync(r->d_scratch, 0, r->scratch_bytes, stream));
-        CU(cudaMemsetAsync(r->d_ranges, 0xff, (size_t)r->tiles_cap * 8 * (r->frame_split ? 2 : 1), stream));    // {begin, ~end} identities for atomicMin (one set per depth slab)
-    }
-    return WS_OK;
 }
 
 // stage 2: depth passes on the V visible splats, tile binning, tile-id passes (+ ranges)
@@ -1131,8 +1160,8 @@ static ws_status enqueue_stage2(ws_renderer *r, cudaStream_t stream)
         // sharded frames: only this rank's band of tile rows (the received rectangles are clipped to it)
         const bool band = r->shard.world > 0;
         a.tile_y0 = band ? r->shard.band_y0[r->shard.rank] : 0u;
-        const uint32_t rows = band ? r->shard.band_y0[r->shard.rank + 1] - r->shard.band_y0[r->shard.rank] : r->h_uniforms.tiles_y;
-        if (rows) CU(launch_composite(a, r->h_uniforms.tiles_x, rows, stream));
+        const uint32_t rows = band ? r->shard.band_y0[r->shard.rank + 1] - r->shard.band_y0[r->shard.rank] : r->h_uniforms.tiles_y / r->views;
+        if (rows) CU(launch_composite(a, r->h_uniforms.tiles_x, rows, stream, r->views));
     }
     if (r->timing) CU(cudaEventRecord(r->ev[EV_NEAR_BLEND], stream));
     return bin_and_tile_sort(2u, 1, EV_BIN2, EV_TSORT2, &r->tile_out_far);
@@ -1198,6 +1227,103 @@ extern "C" ws_status ws_renderer_prepare(ws_renderer *r, ws_pointcloud *pc, cons
         CU(cudaGraphLaunch(r->prep_exec, stream));
     } else {
         st = enqueue_prepare_body(r, pc, stream);
+        if (st != WS_OK) return st;
+    }
+    r->prepared = true;
+    r->last_stream = stream;
+    r->last_n = pc->n;
+    return WS_OK;
+}
+
+// ------------------------------------------------------------------------------------
+// Batches of views of one cloud (DESIGN.md "Batches of views").  The K views are stacked into one "tall" frame: tile
+// (x, y) of view v is tile (v * tiles_y + y) * tiles_x + x.  Stage 1 runs once over the cloud for all views (view-major
+// slots), stage 2 is the single-frame depth sort / binning / tile sort over the K * T tiles, and the compositor runs
+// with gridDim.z = K.  Within each tile the order is (depth key, slot) with slots in Gaussian-index order, exactly as
+// in a single frame, so every view is bit-identical to the same view rendered alone.
+static ws_status enqueue_prepare_views_body(ws_renderer *r, ws_pointcloud *pc, cudaStream_t stream)
+{
+    CU(cudaMemsetAsync(r->d_scratch, 0, r->scratch_bytes, stream));
+    CU(cudaMemsetAsync(r->d_ranges, 0xff, (size_t)r->tiles_cap * 8 * (r->frame_split ? 2 : 1), stream));
+    if (r->timing) CU(cudaEventRecord(r->ev[EV_START], stream));
+    {
+        PreprocessArgs a;
+        a.gaussians = pc->d_gaussians; a.xyz = pc->d_xyz; a.sh_coefs = pc->d_sh; a.covars = pc->d_covars;
+        a.uniforms = r->d_uniforms + 1;                 // the K view-local blocks
+        a.splats = r->d_splats; a.depth_keys = r->d_keys[0]; a.slot_vals = r->d_vals[0]; a.rects = r->d_rects;
+        a.part_counts = r->d_scan_pre; a.part_bases = r->d_part_bases;
+        a.hist = r->d_hist_depth; a.counters = r->d_counters;
+        a.num_views = r->views; a.part_union = r->d_part_union; a.view_visible = r->d_view_visible;
+        CU(launch_preprocess_views(a, r->compressed, r->ctx->sm_count * 8, r->grid_pre_views, stream));
+    }
+    if (r->timing) CU(cudaEventRecord(r->ev[EV_PRE], stream));
+    return enqueue_stage2(r, stream);
+}
+
+extern "C" ws_status ws_renderer_prepare_views(ws_renderer *r, ws_pointcloud *pc, const ws_splatting_args *args,
+                                               uint32_t num_views, void *cuda_stream)
+{
+    if (!r || !pc || !args) return fail(WS_ERR_INVALID_ARGUMENT, "NULL argument");
+    if (num_views == 0 || num_views > WS_MAX_VIEWS) return fail(WS_ERR_INVALID_ARGUMENT, "num_views must be in [1, WS_MAX_VIEWS]");
+    for (uint32_t v = 0; v < num_views; v++) {
+        ws_status st = validate_frame(r, pc, &args[v]);
+        if (st != WS_OK) return st;
+        if (args[v].viewport[0] != args[0].viewport[0] || args[v].viewport[1] != args[0].viewport[1])
+            return fail(WS_ERR_INVALID_ARGUMENT, "the views of a batch must share the viewport");
+    }
+    if (r->shard.world > 0) return fail(WS_ERR_INVALID_ARGUMENT, "batches of views are not supported on a sharded renderer");
+    const uint64_t kn = (uint64_t)num_views * pc->n;
+    if (kn >= (1ull << 30)) return fail(WS_ERR_UNSUPPORTED, "num_views x num_points must be < 2^30 (30-bit look-back counts)");
+    cudaStream_t stream = (cudaStream_t)cuda_stream;
+    CU(cudaSetDevice(r->ctx->device));
+    ws_status st = take_deferred_status(r);
+    if (st != WS_OK) return st;
+    const uint32_t K = num_views, W = args[0].viewport[0], H = args[0].viewport[1];
+    const uint32_t tx = (W + TILE - 1) / TILE, ty = (H + TILE - 1) / TILE;
+    const uint32_t tiles = tx * ty * K;              // < 2^23 for viewports up to 16384 and K <= 8
+    st = decide_split(r, kn, W, H, K);
+    if (st != WS_OK) return st;
+    r->prepared = false; r->rendered = false;
+    st = ensure_capacity(r, (uint32_t)kn, tiles, K);
+    if (st != WS_OK) return st;
+    uint32_t max_deg = 0;
+    for (uint32_t v = 0; v < K; v++) {
+        build_frame_uniforms(r, pc, &args[v], &r->h_views[1 + v]);
+        if (args[v].max_sh_deg > max_deg) max_deg = args[v].max_sh_deg;
+    }
+    FrameUniforms &T = r->h_views[0];                // stages 2-3: view 0's block with K * tiles_y tile rows
+    T = r->h_views[1];
+    T.tiles_y = ty * K;
+    T.rs.max_sh_deg = max_deg;                       // read only by ws_renderer_stats (SH bytes of the batch)
+    r->h_uniforms = T;
+    r->views = K; r->batch = true;
+    r->tile_passes = (tiles > 65536u) ? 3 : ((tiles > 256u) ? 2 : 1);
+    // one upload of the 1 + K blocks in front of the frame (pageable: staged before the call returns)
+    CU(cudaMemcpyAsync(r->d_uniforms, r->h_views, (1 + K) * sizeof(FrameUniforms), cudaMemcpyHostToDevice, stream));
+    if (r->use_graphs && !r->timing) {
+        auto &k = r->views_key;
+        const bool same = r->views_exec && k.pc == pc && k.pc_gen == pc->generation && k.buf_gen == r->buf_generation &&
+                          k.gaussians == pc->d_gaussians && k.scratch == r->d_scratch && k.n == pc->n && k.K == K &&
+                          k.W == W && k.H == H && k.pair_cap == r->pair_cap && k.n_cap == r->n_cap &&
+                          k.split == r->frame_split && k.state == (const void *)r->d_state;
+        if (!same) {
+            if (r->views_exec) { cudaGraphExecDestroy(r->views_exec); r->views_exec = nullptr; }
+            if (!r->cap_stream) CU(cudaStreamCreateWithFlags(&r->cap_stream, cudaStreamNonBlocking));
+            CU(cudaStreamBeginCapture(r->cap_stream, cudaStreamCaptureModeThreadLocal));
+            st = enqueue_prepare_views_body(r, pc, r->cap_stream);
+            cudaGraph_t g = nullptr;
+            cudaError_t e = cudaStreamEndCapture(r->cap_stream, &g);
+            if (st != WS_OK) { if (g) cudaGraphDestroy(g); return st; }
+            if (e != cudaSuccess) return fail_cuda(e, "cudaStreamEndCapture (batch of views)");
+            e = cudaGraphInstantiate(&r->views_exec, g, 0);
+            cudaGraphDestroy(g);
+            if (e != cudaSuccess) { r->views_exec = nullptr; return fail_cuda(e, "cudaGraphInstantiate (batch of views)"); }
+            k.pc = pc; k.pc_gen = pc->generation; k.buf_gen = r->buf_generation; k.gaussians = pc->d_gaussians; k.scratch = r->d_scratch;
+            k.n = pc->n; k.K = K; k.W = W; k.H = H; k.pair_cap = r->pair_cap; k.n_cap = r->n_cap; k.split = r->frame_split; k.state = r->d_state;
+        }
+        CU(cudaGraphLaunch(r->views_exec, stream));
+    } else {
+        st = enqueue_prepare_views_body(r, pc, stream);
         if (st != WS_OK) return st;
     }
     r->prepared = true;
@@ -1416,9 +1542,9 @@ extern "C" ws_status ws_renderer_shard_finish(ws_renderer *r, const uint32_t *ma
 }
 
 static ws_status render_rows(ws_renderer *r, ws_pointcloud *pc, void *dst, size_t row_pitch, const double clear[4],
-                             void *cuda_stream, uint32_t tile_y0, uint32_t tile_rows);
+                             void *cuda_stream, uint32_t tile_y0, uint32_t tile_rows, size_t view_stride = 0);
 static ws_status enqueue_composite(ws_renderer *r, void *dst, size_t row_pitch, const double clear[4], cudaStream_t stream,
-                                   uint32_t tile_y0, uint32_t tile_rows);
+                                   uint32_t tile_y0, uint32_t tile_rows, size_t view_stride = 0);
 static ws_status enqueue_status_copy(ws_renderer *r, cudaStream_t stream);
 
 // The whole sharded frame in ONE call and with NO host-side collective: the count rows, the barrier
@@ -1535,13 +1661,11 @@ extern "C" ws_status ws_renderer_shard_band(const ws_renderer *r, uint32_t *firs
 
 static size_t bytes_per_pixel(ws_format f) { return f == WS_FORMAT_RGBA8_UNORM ? 4 : (f == WS_FORMAT_RGBA16_FLOAT ? 8 : 16); }
 
-static ws_status render_rows(ws_renderer *r, ws_pointcloud *pc, void *dst, size_t row_pitch, const double clear[4],
-                             void *cuda_stream, uint32_t tile_y0, uint32_t tile_rows);
-
 extern "C" ws_status ws_renderer_render(ws_renderer *r, ws_pointcloud *pc, void *dst, size_t row_pitch,
                                         const double clear[4], void *cuda_stream)
 {
     if (r && r->shard.world > 1) return fail(WS_ERR_INVALID_ARGUMENT, "sharded renderer: use ws_renderer_render_band");
+    if (r && r->batch) return fail(WS_ERR_INVALID_ARGUMENT, "the prepared frame is a batch of views: use ws_renderer_render_views");
     return render_rows(r, pc, dst, row_pitch, clear, cuda_stream, 0, r ? r->h_uniforms.tiles_y : 0);
 }
 
@@ -1583,7 +1707,7 @@ extern "C" ws_status ws_renderer_shard_download(ws_renderer *r, void *dst_host, 
 
 // stage 3 launch only (capturable): the compositor over tile rows [tile_y0, tile_y0 + tile_rows) into dst
 static ws_status enqueue_composite(ws_renderer *r, void *dst, size_t row_pitch, const double clear[4], cudaStream_t stream,
-                                   uint32_t tile_y0, uint32_t tile_rows)
+                                   uint32_t tile_y0, uint32_t tile_rows, size_t view_stride)
 {
     const FrameUniforms &U = r->h_uniforms;
     CompositeArgs a;
@@ -1594,12 +1718,12 @@ static ws_status enqueue_composite(ws_renderer *r, void *dst, size_t row_pitch, 
         a.mode = 2; a.state = r->d_state; a.tile_done = r->d_tile_done;
     }
     a.uniforms = r->d_uniforms; a.dst = dst; a.row_pitch = (uint32_t)row_pitch; a.format = (int)r->format;
-    a.tile_y0 = tile_y0; a.active_cull = active_cull_default();
+    a.tile_y0 = tile_y0; a.active_cull = active_cull_default(); a.view_stride = view_stride;
     a.signal_flag = r->shard.pending_signal; a.signal_epoch = r->shard.d_epoch; a.done_counter = &r->d_counters->composite_done;
     r->shard.pending_signal = nullptr;
     for (int i = 0; i < 4; i++) a.clear[i] = clear ? (float)clear[i] : 0.f;
     if (r->timing) CU(cudaEventRecord(r->ev[EV_BLEND0], stream));
-    if (tile_rows) CU(launch_composite(a, U.tiles_x, tile_rows, stream));
+    if (tile_rows) CU(launch_composite(a, U.tiles_x, tile_rows, stream, r->views));
     if (r->timing) CU(cudaEventRecord(r->ev[EV_BLEND1], stream));
     return WS_OK;
 }
@@ -1615,7 +1739,7 @@ static ws_status enqueue_status_copy(ws_renderer *r, cudaStream_t stream)
 }
 
 static ws_status render_rows(ws_renderer *r, ws_pointcloud *pc, void *dst, size_t row_pitch, const double clear[4],
-                             void *cuda_stream, uint32_t tile_y0, uint32_t tile_rows)
+                             void *cuda_stream, uint32_t tile_y0, uint32_t tile_rows, size_t view_stride)
 {
     if (!r || !pc || !dst) return fail(WS_ERR_INVALID_ARGUMENT, "NULL argument");
     if (!r->prepared) return fail(WS_ERR_NOT_PREPARED, "prepare() must precede render()");
@@ -1626,7 +1750,7 @@ static ws_status render_rows(ws_renderer *r, ws_pointcloud *pc, void *dst, size_
     if (((uintptr_t)dst % bpp) != 0) return fail(WS_ERR_INVALID_ARGUMENT, "dst is not aligned to the pixel size");
     cudaStream_t stream = (cudaStream_t)cuda_stream;
     CU(cudaSetDevice(r->ctx->device));
-    ws_status st = enqueue_composite(r, dst, row_pitch, clear, stream, tile_y0, tile_rows);
+    ws_status st = enqueue_composite(r, dst, row_pitch, clear, stream, tile_y0, tile_rows, view_stride);
     if (st != WS_OK) return st;
     st = enqueue_status_copy(r, stream);
     if (st != WS_OK) return st;
@@ -1640,6 +1764,7 @@ extern "C" ws_status ws_renderer_render_to_host(ws_renderer *r, ws_pointcloud *p
 {
     if (!r || !pc || !dst_host) return fail(WS_ERR_INVALID_ARGUMENT, "NULL argument");
     if (!r->prepared) return fail(WS_ERR_NOT_PREPARED, "prepare() must precede render()");
+    if (r->batch) return fail(WS_ERR_INVALID_ARGUMENT, "the prepared frame is a batch of views: use ws_renderer_render_views_to_host");
     const FrameUniforms &U = r->h_uniforms;
     const size_t bpp = bytes_per_pixel(r->format);
     const size_t tight = (size_t)U.width * bpp;
@@ -1656,6 +1781,66 @@ extern "C" ws_status ws_renderer_render_to_host(ws_renderer *r, ws_pointcloud *p
     cudaStream_t stream = (cudaStream_t)cuda_stream;
     if (row_pitch == tight) CU(cudaMemcpyAsync(dst_host, r->d_frame, need, cudaMemcpyDeviceToHost, stream));
     else CU(cudaMemcpy2DAsync(dst_host, row_pitch, r->d_frame, tight, tight, U.height, cudaMemcpyDeviceToHost, stream));
+    return WS_OK;
+}
+
+static ws_status check_views_target(ws_renderer *r, ws_pointcloud *pc, const void *dst, size_t row_pitch, size_t view_stride)
+{
+    if (!r || !pc || !dst) return fail(WS_ERR_INVALID_ARGUMENT, "NULL argument");
+    if (!r->prepared) return fail(WS_ERR_NOT_PREPARED, "prepare_views() must precede render_views()");
+    if (!r->batch) return fail(WS_ERR_INVALID_ARGUMENT, "the prepared frame is a single view: use ws_renderer_render");
+    if (r->shard.world > 0) return fail(WS_ERR_INVALID_ARGUMENT, "batches of views are not supported on a sharded renderer");
+    const size_t bpp = bytes_per_pixel(r->format);
+    if (view_stride < (size_t)r->h_uniforms.height * row_pitch || (view_stride % bpp) != 0)
+        return fail(WS_ERR_INVALID_ARGUMENT, "view_stride_bytes smaller than height * row_pitch_bytes or not a multiple of the pixel size");
+    return WS_OK;
+}
+
+extern "C" ws_status ws_renderer_render_views(ws_renderer *r, ws_pointcloud *pc, void *dst, size_t row_pitch,
+                                              size_t view_stride, const double clear[4], void *cuda_stream)
+{
+    ws_status st = check_views_target(r, pc, dst, row_pitch, view_stride);
+    if (st != WS_OK) return st;
+    return render_rows(r, pc, dst, row_pitch, clear, cuda_stream, 0, r->h_uniforms.tiles_y / r->views, view_stride);
+}
+
+extern "C" ws_status ws_renderer_render_views_to_host(ws_renderer *r, ws_pointcloud *pc, void *dst_host, size_t row_pitch,
+                                                      size_t view_stride, const double clear[4], void *cuda_stream)
+{
+    ws_status st = check_views_target(r, pc, dst_host, row_pitch, view_stride);
+    if (st != WS_OK) return st;
+    const FrameUniforms &U = r->h_uniforms;
+    const size_t tight = (size_t)U.width * bytes_per_pixel(r->format);
+    if (row_pitch < tight) return fail(WS_ERR_INVALID_ARGUMENT, "row_pitch_bytes too small");
+    const size_t view_bytes = tight * U.height, need = view_bytes * r->views;
+    CU(cudaSetDevice(r->ctx->device));
+    if (r->frame_bytes < need) {
+        cudaFree(r->d_frame); r->d_frame = nullptr; r->frame_bytes = 0;
+        CU(cudaMalloc(&r->d_frame, need));
+        r->frame_bytes = need;
+    }
+    st = ws_renderer_render_views(r, pc, r->d_frame, tight, view_bytes, clear, cuda_stream);
+    if (st != WS_OK) return st;
+    cudaStream_t stream = (cudaStream_t)cuda_stream;
+    if (row_pitch == tight && view_stride == view_bytes) {
+        CU(cudaMemcpyAsync(dst_host, r->d_frame, need, cudaMemcpyDeviceToHost, stream));
+    } else {
+        for (uint32_t v = 0; v < r->views; v++)
+            CU(cudaMemcpy2DAsync(static_cast<uint8_t *>(dst_host) + v * view_stride, row_pitch, static_cast<uint8_t *>(r->d_frame) + v * view_bytes,
+                                 tight, tight, U.height, cudaMemcpyDeviceToHost, stream));
+    }
+    return WS_OK;
+}
+
+extern "C" ws_status ws_renderer_views_num_visible_points(ws_renderer *r, uint32_t *out, uint32_t count)
+{
+    if (!r || !out) return fail(WS_ERR_INVALID_ARGUMENT, "NULL argument");
+    if (!r->prepared) return fail(WS_ERR_NOT_PREPARED, "no frame prepared");
+    if (!r->batch) return fail(WS_ERR_INVALID_ARGUMENT, "the prepared frame is not a batch of views");
+    if (count < r->views) return fail(WS_ERR_INVALID_ARGUMENT, "count is smaller than the number of views");
+    CU(cudaSetDevice(r->ctx->device));
+    CU(cudaStreamSynchronize(r->last_stream));
+    CU(cudaMemcpy(out, r->d_view_visible, r->views * sizeof(uint32_t), cudaMemcpyDeviceToHost));
     return WS_OK;
 }
 
@@ -1707,18 +1892,21 @@ extern "C" ws_status ws_renderer_stats(ws_renderer *r, ws_frame_stats *s)
         s->ms_sort = s->ms_depth_sort + s->ms_binning + s->ms_tile_sort;
         cudaGetLastError();
     }
+    // a batch of K views (DESIGN.md "Batches of views"): V = sum of the V_v, T = K x tiles of one view, K x W x H pixels;
+    // the cloud is read once and the SH of a Gaussian at most once (charged as min(V, N) at the batch's highest degree)
     const uint64_t N = r->last_n, V = c.num_visible;
     const uint64_t P = s->num_pairs < r->pair_cap ? s->num_pairs : r->pair_cap;
     const uint64_t T = s->num_tiles;
+    const uint64_t px = (uint64_t)U.width * U.height * r->views;
     const uint64_t rec = r->compressed ? 24 : 28;
     const uint64_t ncoef = (uint64_t)(U.rs.max_sh_deg + 1) * (U.rs.max_sh_deg + 1);
     const uint64_t shb = r->compressed ? (12 + 3 * ncoef) : (U.rs.max_sh_deg >= 3 ? 96 : (U.rs.max_sh_deg == 2 ? 64 : 32));
-    s->bytes_preprocess = N * 12 + N * rec + V * shb + V * (20 + 4 + 4 + 8);   // count (xyz plane) + main
+    s->bytes_preprocess = N * 12 + N * rec + (V < N ? V : N) * shb + V * (20 + 4 + 4 + 8);   // count (xyz plane) + main
     s->bytes_sort = (uint64_t)r->depth_passes * V * 16 + V * 12 + P * 8 + (uint64_t)r->tile_passes * P * 16 + T * 8;
-    s->bytes_blend = P * 24 + T * 8 + (uint64_t)U.width * U.height * bytes_per_pixel(r->format);
+    s->bytes_blend = P * 24 + T * 8 + px * bytes_per_pixel(r->format);
     if (r->frame_split) {                                         // the far slab re-reads the slots + rectangles, the state goes out and in
         s->bytes_sort += (V - V / 4) * 12;
-        s->bytes_blend += T * 8 + (uint64_t)U.width * U.height * 32;
+        s->bytes_blend += T * 8 + px * 32;
     }
     if (c.error_flags) return fail(WS_ERR_CUDA, (c.error_flags & 2u) ? "sharded frame: receive capacity exceeded" : ((c.error_flags & 4u) ? "sharded frame: a peer never arrived" : "internal: decoupled look-back watchdog fired"));
     if (c.pair_overflow) return fail(WS_ERR_PAIR_OVERFLOW, "pair capacity exceeded; raise it with ws_renderer_set_pair_capacity");
@@ -1729,6 +1917,7 @@ extern "C" ws_status ws_renderer_read_buffer(ws_renderer *r, ws_buffer_id which,
 {
     if (!r || !dst) return fail(WS_ERR_INVALID_ARGUMENT, "NULL argument");
     if (!r->prepared) return fail(WS_ERR_NOT_PREPARED, "no frame prepared");
+    if (r->batch) return fail(WS_ERR_UNSUPPORTED, "intermediate buffers of a batch of views cannot be read back");
     FrameCounters c;
     ws_status st = read_counters(r, &c);
     if (st != WS_OK) return st;
@@ -1791,12 +1980,14 @@ extern "C" ws_status ws_renderer_read_buffer(ws_renderer *r, ws_buffer_id which,
 extern "C" ws_status ws_renderer_camera_uniform(const ws_renderer *r, float out68[68])
 {
     if (!r || !out68) return fail(WS_ERR_INVALID_ARGUMENT, "NULL argument");
+    if (r->batch) return fail(WS_ERR_UNSUPPORTED, "the prepared frame is a batch of views");
     memcpy(out68, &r->h_uniforms.cam, sizeof(CameraUniform));
     return WS_OK;
 }
 extern "C" ws_status ws_renderer_settings_uniform(const ws_renderer *r, void *out80)
 {
     if (!r || !out80) return fail(WS_ERR_INVALID_ARGUMENT, "NULL argument");
+    if (r->batch) return fail(WS_ERR_UNSUPPORTED, "the prepared frame is a batch of views");
     memcpy(out80, &r->h_uniforms.rs, sizeof(RenderSettings));
     return WS_OK;
 }

@@ -91,7 +91,7 @@ composite_kernel(CompositeArgs a)
     const unsigned tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
     const uint32_t W = a.uniforms->width, H = a.uniforms->height;
     const uint32_t tile_x = blockIdx.x, tile_y = blockIdx.y + a.tile_y0;
-    const uint32_t tile = tile_y * gridDim.x + tile_x;
+    const uint32_t tile = (blockIdx.z * gridDim.y + tile_y) * gridDim.x + tile_x;     // z > 0 only in batches (tile_y0 = 0)
     uint2 range = a.ranges[tile];
     range.y = ~range.y;                                  // stored complemented (atomicMin in the sort's last pass)
     if (range.y <= range.x) range.x = range.y = 0u;      // untouched tile
@@ -114,7 +114,7 @@ composite_kernel(CompositeArgs a)
     float T = inside ? 1.f : 0.f, cr = 0.f, cg = 0.f, cb = 0.f;
     if (MODE == 2) {
         if (inside) {
-            const float4 st = a.state[(size_t)py * W + px];
+            const float4 st = a.state[((size_t)blockIdx.z * H + py) * W + px];
             cr = st.x; cg = st.y; cb = st.z; T = st.w;
         }
         if (a.tile_done[tile]) range.x = range.y = 0u;   // saturated by the near slab: nothing of the far slab can show
@@ -209,7 +209,7 @@ composite_kernel(CompositeArgs a)
     }
 
     if (MODE == 1) {
-        if (inside) a.state[(size_t)py * W + px] = make_float4(cr, cg, cb, T);
+        if (inside) a.state[((size_t)blockIdx.z * H + py) * W + px] = make_float4(cr, cg, cb, T);
         const int all_done = __syncthreads_and(T == 0.f ? 1 : 0);
         if (tid == 0) a.tile_done[tile] = (uint8_t)(all_done ? 1 : 0);
         return;
@@ -217,7 +217,7 @@ composite_kernel(CompositeArgs a)
     if (inside) {
         const float r = cr + a.clear[0] * T, g = cg + a.clear[1] * T, b = cb + a.clear[2] * T;
         const float al = (1.f - T) + a.clear[3] * T;
-        uint8_t *row = reinterpret_cast<uint8_t *>(a.dst) + (size_t)(py - a.tile_y0 * TILE) * a.row_pitch;
+        uint8_t *row = reinterpret_cast<uint8_t *>(a.dst) + blockIdx.z * a.view_stride + (size_t)(py - a.tile_y0 * TILE) * a.row_pitch;
         if (FORMAT == 2) {
             reinterpret_cast<float4 *>(row)[px] = make_float4(r, g, b, al);
         } else if (FORMAT == 1) {
@@ -243,9 +243,9 @@ composite_kernel(CompositeArgs a)
 
 }  // namespace
 
-cudaError_t launch_composite(const CompositeArgs &a, uint32_t tiles_x, uint32_t tiles_y, cudaStream_t stream)
+cudaError_t launch_composite(const CompositeArgs &a, uint32_t tiles_x, uint32_t tiles_y, cudaStream_t stream, uint32_t views)
 {
-    dim3 grid(tiles_x, tiles_y);
+    dim3 grid(tiles_x, tiles_y, views);
     if (a.mode == 1) {
         composite_kernel<2, 1><<<grid, CB_THREADS, 0, stream>>>(a);          // no pixels are written: the format is irrelevant
     } else if (a.mode == 2) {

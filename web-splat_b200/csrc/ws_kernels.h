@@ -24,9 +24,17 @@ struct PreprocessArgs {
     uint32_t *part_bases;         // ceil(N/256): exclusive scan of part_counts (scan kernel)
     uint32_t *hist;               // 4 x 256 depth-key digit histograms (zeroed per frame)
     FrameCounters *counters;
+    // batches of views only (launch_preprocess_views): `uniforms` then points at num_views view-local blocks,
+    // part_counts / part_bases hold num_views x ceil(N/256) entries (view-major)
+    uint32_t num_views;
+    uint32_t *part_union;         // ceil(N/256): Gaussians of the partition that survive in at least one view
+    uint32_t *view_visible;       // out: num_views per-view survivor counts V_v
 };
 cudaError_t launch_preprocess(const PreprocessArgs &a, bool compressed, int grid_count, int grid_main, cudaStream_t stream);
 int preprocess_blocks_per_sm(bool compressed);
+constexpr uint32_t MAX_VIEWS = 8;  // views per batch (WS_MAX_VIEWS)
+cudaError_t launch_preprocess_views(const PreprocessArgs &a, bool compressed, int grid_count, int grid_main, cudaStream_t stream);
+int preprocess_views_blocks_per_sm(bool compressed);
 
 // ---- onesweep radix sort of (u32 key, u32 value) pairs ---------------------------
 constexpr int SORT_THREADS = 256;
@@ -96,10 +104,13 @@ struct CompositeArgs {
     // "saturated" flag out, no pixels; 2 = far slab, state in, final pixels out
     int mode;
     int active_cull;              // per-warp cull against the bounding box of the still-unsaturated pixels (result-neutral)
-    float4 *state;                // W x H
+    float4 *state;                // W x H per view
     uint8_t *tile_done;           // T
+    // batches of views: block z composites view z, whose tiles follow the tiles of views 0..z-1 ("tall" frame of
+    // z * tiles_y + y rows), whose state starts at z * W * H and whose pixels start at dst + z * view_stride
+    uint64_t view_stride;         // bytes
 };
-cudaError_t launch_composite(const CompositeArgs &a, uint32_t tiles_x, uint32_t tiles_y, cudaStream_t stream);
+cudaError_t launch_composite(const CompositeArgs &a, uint32_t tiles_x, uint32_t tiles_y, cudaStream_t stream, uint32_t views = 1);
 
 // ---- file-format ingest (ingest.cu) ---------------------------------------------------------------------------
 struct PlyConvertArgs {

@@ -215,14 +215,49 @@ def render_resolution(width, height):
     return int(width), int(height)
 
 
-def render_views(ws, ctx, renderer, pc, cameras, img_out, split, on_frame=None):
+def _batches(cameras, batch):
+    """Consecutive cameras of equal render resolution, in groups of at most `batch`: [(first index, [cameras])]."""
+    groups = []
+    for i, s in enumerate(cameras):
+        res = render_resolution(s.width, s.height)
+        if groups and len(groups[-1][2]) < batch and groups[-1][1] == res:
+            groups[-1][2].append(s)
+        else:
+            groups.append((i, res, [s]))
+    return [(i0, cams) for i0, _, cams in groups]
+
+
+def render_views(ws, ctx, renderer, pc, cameras, img_out, split, on_frame=None, batch=1):
     """bin/render.rs:33-127: renders every camera of one split to `<img_out>/<split>/<index:05>.png`.
-    The next view's prepare+render is enqueued while the previous frame is being encoded to PNG."""
+    The next view's prepare+render is enqueued while the previous frame is being encoded to PNG.
+    batch > 1 renders consecutive cameras of equal resolution together, up to `batch` (<= ws.MAX_VIEWS) per
+    prepare_views / render_views; the images are bit-identical to batch = 1."""
     import torch
     out_dir = os.path.join(img_out, split)
     os.makedirs(out_dir, exist_ok=True)
     bbox = pc.bbox()
     paths = []
+    if batch > 1:
+        for i0, cams in _batches(cameras, batch):
+            W, H = render_resolution(cams[0].width, cams[0].height)
+            args = []
+            for s in cams:
+                cam = s.to_perspective(ws)
+                cam.fit_near_far(bbox)
+                args.append(ws.SplattingArgs(cam, (W, H), gaussian_scaling=1.0, max_sh_deg=pc.sh_deg(), walltime=100.0))
+            renderer.prepare_views(None, pc, args)
+            host = torch.empty((len(cams), H, W, 4), dtype=torch.float16).pin_memory()
+            renderer.render_views_to_host(host, pc, clear=(0.0, 0.0, 0.0, 0.0))
+            torch.cuda.synchronize()
+            frames = host.numpy()
+            for j, s in enumerate(cams):
+                if on_frame is not None:
+                    on_frame(i0 + j, s, frames[j])
+                path = os.path.join(out_dir, "%05d.png" % (i0 + j))
+                with open(path, "wb") as f:
+                    f.write(png_bytes(frame_to_rgba8(frames[j])))
+                paths.append(path)
+        return paths
     for i, s in enumerate(cameras):
         W, H = render_resolution(s.width, s.height)
         cam = s.to_perspective(ws)
