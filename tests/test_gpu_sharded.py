@@ -57,6 +57,13 @@ def test_sharded_world1_equals_plain(ws, orc, ctx):
     st = sh.stats()
     # only splats that touch at least one tile are routed, so the received count can be below V
     assert st["num_visible"] <= plain.stats()["num_visible"] and st["num_pairs"] == plain.stats()["num_pairs"]
+    # timing off: the frame runs as a CUDA graph, one per frame-buffer parity (two captures, then a replay)
+    sh.r.set_timing(False)
+    for _ in range(3):
+        host.zero_()
+        sh.frame_peer(args, host=host)
+        torch.cuda.synchronize()
+        assert torch.equal(host, t.cpu())
     # two frames in flight through the gated path (world 1: the gates wait on this rank's own flags)
     pipe = ws.ShardedPipeline(ws, ctx, ws.FORMAT_RGBA32_FLOAT, 3, False, pc, cloud["num_points"], (W, H), depth=2)
     hosts = [torch.zeros((H, W, 4), dtype=torch.float32).pin_memory() for _ in range(4)]

@@ -701,6 +701,17 @@ struct ShardState {
     int phase = 0;
 };
 
+// What a captured prepare() graph depends on besides the sizes the kernels read from device memory
+struct PrepKey {
+    const ws_pointcloud *pc; uint64_t pc_gen, buf_gen; const void *gaussians, *scratch, *state; uint32_t n, K, W, H, pair_cap, n_cap; bool split;
+    bool operator==(const PrepKey &o) const
+    {
+        return pc == o.pc && pc_gen == o.pc_gen && buf_gen == o.buf_gen && gaussians == o.gaussians && scratch == o.scratch &&
+               state == o.state && n == o.n && K == o.K && W == o.W && H == o.H && pair_cap == o.pair_cap && n_cap == o.n_cap &&
+               split == o.split;
+    }
+};
+
 struct ws_renderer {
     ws_context *ctx;
     ws_format format;
@@ -729,7 +740,7 @@ struct ws_renderer {
     void *d_frame = nullptr; size_t frame_bytes = 0;
 
     // launch geometry
-    int grid_pre = 0, grid_sort = 0, grid_bin = 0;
+    int grid_pre[2] = {0, 0}, grid_sort = 0, grid_bin = 0;     // grid_pre[batch]: single frames / batches of views
 
     // frame state
     FrameUniforms h_uniforms;
@@ -752,7 +763,9 @@ struct ws_renderer {
     uint32_t *d_keep4 = nullptr;           // far slab: one byte per splat, written by bin_count, read by bin_expand
     int tile_out_far = 0;
     cudaStream_t cap_stream = nullptr;
-    cudaGraphExec_t prep_exec = nullptr;
+    // [batch]: a graph per mode, so a renderer that alternates single frames and batches never recaptures
+    cudaGraphExec_t prep_exec[2] = {nullptr, nullptr};
+    PrepKey prep_key[2] = {};
     // deferred frame status: render() copies {V, P, pair_overflow, error_flags} of its frame into a ring of pinned slots;
     // the NEXT prepare()/render() whose predecessor's copy has completed returns that frame's error once
     // (WS_ERR_PAIR_OVERFLOW / WS_ERR_CUDA) instead of WS_OK -- no synchronisation; ws_renderer_stats() consumes them too
@@ -762,17 +775,14 @@ struct ws_renderer {
     bool flags_pending[FLAG_SLOTS] = {};
     int flag_next = 0;
     uint64_t buf_generation = 0;           // bumped whenever a buffer a captured graph points into is (re)allocated
-    struct { const ws_pointcloud *pc; uint64_t pc_gen, buf_gen; const void *gaussians, *scratch, *state; uint32_t n, W, H, pair_cap, n_cap; bool split; } prep_key = {};
-    // batch of views (ws_renderer_prepare_views): d_uniforms holds 1 + WS_MAX_VIEWS blocks, [0] = the "tall" frame of
-    // K * tiles_y tile rows that stages 2-3 see, [1 + v] = view v's own block for stage 1
+    // d_uniforms holds 1 + WS_MAX_VIEWS blocks: [1 + v] = view v's own block, read by stage 1 (a single frame has K = 1
+    // view), and [0] = the frame that stages 2-3 see, for a batch of views (ws_renderer_prepare_views) the "tall" frame
+    // of K * tiles_y tile rows
     uint32_t views = 1;                    // views of the prepared frame
     bool batch = false;                    // the prepared frame is a batch (prepare_views)
     uint32_t *d_view_visible = nullptr;    // WS_MAX_VIEWS per-view survivor counts (in d_scratch)
     uint32_t *d_part_union = nullptr;      // per 256-Gaussian partition: survivors in any view (in d_scratch)
-    int grid_pre_views = 0;
     FrameUniforms h_views[1 + WS_MAX_VIEWS];
-    cudaGraphExec_t views_exec = nullptr;  // its own graph, so alternating single frames and batches never recaptures
-    struct { const ws_pointcloud *pc; uint64_t pc_gen, buf_gen; const void *gaussians, *scratch, *state; uint32_t n, K, W, H, pair_cap, n_cap; bool split; } views_key = {};
 };
 static_assert(WS_MAX_VIEWS == MAX_VIEWS, "views per batch");
 
@@ -802,8 +812,7 @@ extern "C" void ws_renderer_destroy(ws_renderer *r)
     if (r->ev_ok) for (int i = 0; i < EV_COUNT; i++) cudaEventDestroy(r->ev[i]);
     for (int i = 0; i < ws_renderer::FLAG_SLOTS; i++) if (r->ev_flags[i]) cudaEventDestroy(r->ev_flags[i]);
     if (r->h_flags) cudaFreeHost(r->h_flags);
-    if (r->prep_exec) cudaGraphExecDestroy(r->prep_exec);
-    if (r->views_exec) cudaGraphExecDestroy(r->views_exec);
+    for (int i = 0; i < 2; i++) if (r->prep_exec[i]) cudaGraphExecDestroy(r->prep_exec[i]);
     if (r->cap_stream) cudaStreamDestroy(r->cap_stream);
     delete r;
 }
@@ -829,13 +838,12 @@ extern "C" ws_status ws_renderer_create(ws_context *ctx, ws_format fmt, uint32_t
     for (int i = 0; i < ws_renderer::FLAG_SLOTS && e == cudaSuccess; i++) e = cudaEventCreateWithFlags(&r->ev_flags[i], cudaEventDisableTiming);
     if (e != cudaSuccess) { ws_status s = fail_cuda(e, "deferred-status slots"); ws_renderer_destroy(r); return s; }
     // persistent grids: one wave of resident CTAs
-    r->grid_pre = ctx->sm_count * preprocess_blocks_per_sm(r->compressed);
+    for (int b = 0; b < 2; b++) r->grid_pre[b] = ctx->sm_count * preprocess_blocks_per_sm(r->compressed, b != 0);
     r->grid_sort = ctx->sm_count * sort_pass_blocks_per_sm();
     r->grid_bin = ctx->sm_count * binning_blocks_per_sm();
-    r->grid_pre_views = ctx->sm_count * preprocess_views_blocks_per_sm(r->compressed);
     {   // A/B knobs (profiles/): fewer resident CTAs per SM for the persistent kernels leave room for the other frame's kernels
         auto per_sm = [&](const char *name, int cur) { const char *e = getenv(name); const int k = e ? atoi(e) : 0; return (k >= 1 && k * ctx->sm_count < cur) ? k * ctx->sm_count : cur; };
-        r->grid_pre = per_sm("WS_PRE_CTAS_PER_SM", r->grid_pre);
+        for (int b = 0; b < 2; b++) r->grid_pre[b] = per_sm("WS_PRE_CTAS_PER_SM", r->grid_pre[b]);
         r->grid_sort = per_sm("WS_SORT_CTAS_PER_SM", r->grid_sort);
         r->grid_bin = per_sm("WS_BIN_CTAS_PER_SM", r->grid_bin);
     }
@@ -1033,23 +1041,32 @@ static ws_status decide_split(ws_renderer *r, uint64_t points_here, uint32_t W, 
 
 static void build_frame_uniforms(ws_renderer *r, ws_pointcloud *pc, const ws_splatting_args *args, FrameUniforms *out);
 
-// uniforms + per-frame clears (everything before stage 1)
-static ws_status begin_frame(ws_renderer *r, ws_pointcloud *pc, const ws_splatting_args *args, uint32_t capacity_points, cudaStream_t stream,
-                            bool with_clears = true)
+// uniforms + per-frame clears (everything before stage 1) of a frame of K views that share the viewport (sharded
+// frames: K = 1) and `capacity_points` splats.  A batch of K views is stacked into one "tall" frame of K * T tiles.
+static ws_status begin_frame(ws_renderer *r, ws_pointcloud *pc, const ws_splatting_args *args, uint32_t K, bool batch,
+                             uint32_t capacity_points, cudaStream_t stream, bool with_clears = true)
 {
-    const uint32_t W = args->viewport[0], H = args->viewport[1];
+    const uint32_t W = args[0].viewport[0], H = args[0].viewport[1];
     const uint32_t tx = (W + TILE - 1) / TILE, ty = (H + TILE - 1) / TILE;
-    const uint32_t tiles = tx * ty;
-    r->prepared = false; r->rendered = false; r->batch = false; r->views = 1;
-    ws_status st = ensure_capacity(r, capacity_points, tiles);
+    const uint32_t tiles = tx * ty * K;              // < 2^23 for viewports up to 16384 and K <= 8
+    r->prepared = false; r->rendered = false; r->batch = batch; r->views = K;
+    ws_status st = ensure_capacity(r, capacity_points, tiles, K);
     if (st != WS_OK) return st;
 
-    FrameUniforms &U = r->h_uniforms;
-    build_frame_uniforms(r, pc, args, &U);
+    uint32_t max_deg = 0;
+    for (uint32_t v = 0; v < K; v++) {
+        build_frame_uniforms(r, pc, &args[v], &r->h_views[1 + v]);
+        if (args[v].max_sh_deg > max_deg) max_deg = args[v].max_sh_deg;
+    }
+    FrameUniforms &T = r->h_views[0];                // stages 2-3: view 0's block with K * tiles_y tile rows
+    T = r->h_views[1];
+    T.tiles_y = ty * K;
+    T.rs.max_sh_deg = max_deg;                       // read only by ws_renderer_stats (SH bytes of the batch)
+    r->h_uniforms = T;
     r->tile_passes = (tiles > 65536u) ? 3 : ((tiles > 256u) ? 2 : 1);
 
-    // pageable source: the runtime stages the 0.5 KB before returning, so h_uniforms may be reused
-    CU(cudaMemcpyAsync(r->d_uniforms, &U, sizeof U, cudaMemcpyHostToDevice, stream));
+    // one upload of the 1 + K blocks in front of the frame (pageable: staged before the call returns)
+    CU(cudaMemcpyAsync(r->d_uniforms, r->h_views, (1 + K) * sizeof(FrameUniforms), cudaMemcpyHostToDevice, stream));
     if (with_clears) {
         CU(cudaMemsetAsync(r->d_scratch, 0, r->scratch_bytes, stream));
         CU(cudaMemsetAsync(r->d_ranges, 0xff, (size_t)r->tiles_cap * 8 * (r->frame_split ? 2 : 1), stream));    // {begin, ~end} identities for atomicMin (one set per depth slab)
@@ -1167,97 +1184,102 @@ static ws_status enqueue_stage2(ws_renderer *r, cudaStream_t stream)
     return bin_and_tile_sort(2u, 1, EV_BIN2, EV_TSORT2, &r->tile_out_far);
 }
 
-// clears + stage 1 + stage 2 of the plain (single-GPU) frame, on `stream`
-static ws_status enqueue_prepare_body(ws_renderer *r, ws_pointcloud *pc, cudaStream_t stream)
+// Stage-1 arguments of the frame begin_frame() set up: the view blocks d_uniforms[1..K] in, the depth sort's input out
+static PreprocessArgs stage1_args(const ws_renderer *r, const ws_pointcloud *pc)
 {
-    const FrameUniforms &U = r->h_uniforms;
-    CU(cudaMemsetAsync(r->d_scratch, 0, r->scratch_bytes, stream));
-    CU(cudaMemsetAsync(r->d_ranges, 0xff, (size_t)r->tiles_cap * 8 * (r->frame_split ? 2 : 1), stream));    // {begin, ~end} identities for atomicMin
-    if (r->timing) CU(cudaEventRecord(r->ev[EV_START], stream));
-    {   // ---- stage 1
-        PreprocessArgs a;
-        a.gaussians = pc->d_gaussians; a.xyz = pc->d_xyz; a.sh_coefs = pc->d_sh; a.covars = pc->d_covars;
-        a.uniforms = r->d_uniforms;
-        a.splats = r->d_splats; a.depth_keys = r->d_keys[0]; a.slot_vals = r->d_vals[0]; a.rects = r->d_rects;
-        a.part_counts = r->d_scan_pre; a.part_bases = r->d_part_bases;
-        a.hist = r->d_hist_depth; a.counters = r->d_counters;
-        CU(launch_preprocess(a, r->compressed, r->ctx->sm_count * 8, r->grid_pre, stream));
-    }
-    if (r->timing) CU(cudaEventRecord(r->ev[EV_PRE], stream));
-    return enqueue_stage2(r, stream);
+    PreprocessArgs a;
+    a.gaussians = pc->d_gaussians; a.xyz = pc->d_xyz; a.sh_coefs = pc->d_sh; a.covars = pc->d_covars;
+    a.uniforms = r->d_uniforms + 1;
+    a.splats = r->d_splats; a.depth_keys = r->d_keys[0]; a.slot_vals = r->d_vals[0]; a.rects = r->d_rects;
+    a.part_counts = r->d_scan_pre; a.part_bases = r->d_part_bases;
+    a.hist = r->d_hist_depth; a.counters = r->d_counters;
+    a.num_views = r->views; a.part_union = r->d_part_union; a.view_visible = r->d_view_visible;
+    return a;
 }
 
-extern "C" ws_status ws_renderer_prepare(ws_renderer *r, ws_pointcloud *pc, const ws_splatting_args *args, void *cuda_stream)
+// Runs body() on `stream`, or -- with CUDA graphs on and timing off -- launches the graph in `exec`, first capturing it
+// from body() when there is none or `same` is false (its key changed); *captured then tells the caller to store the
+// new key.  `label` ends the error messages.
+template <class Body>
+static ws_status run_graph(ws_renderer *r, cudaGraphExec_t &exec, bool same, bool *captured, const char *label,
+                           cudaStream_t stream, Body &&body)
 {
-    ws_status st = validate_frame(r, pc, args);
-    if (st != WS_OK) return st;
-    if (r->shard.world > 1) return fail(WS_ERR_INVALID_ARGUMENT, "renderer is configured for sharding: use ws_renderer_shard_begin/exchange/finish");
-    cudaStream_t stream = (cudaStream_t)cuda_stream;
-    CU(cudaSetDevice(r->ctx->device));
-    st = take_deferred_status(r);
-    if (st != WS_OK) return st;
-    st = decide_split(r, pc->n, args->viewport[0], args->viewport[1]);
-    if (st != WS_OK) return st;
-    st = begin_frame(r, pc, args, pc->n, stream, /*with_clears=*/false);     // uniforms only; capacities may (re)allocate
-    if (st != WS_OK) return st;
-    if (r->use_graphs && !r->timing) {
-        // One CUDA graph per (cloud, viewport, capacities): 2 memsets + 14 kernels become one launch.  Every kernel
-        // reads its sizes (N, V, P) from device memory, so the graph is independent of the frame's content.
-        const FrameUniforms &U = r->h_uniforms;
-        auto &k = r->prep_key;
-        const bool same = r->prep_exec && k.pc == pc && k.pc_gen == pc->generation && k.buf_gen == r->buf_generation &&
-                          k.gaussians == pc->d_gaussians && k.scratch == r->d_scratch && k.n == pc->n &&
-                          k.W == U.width && k.H == U.height && k.pair_cap == r->pair_cap && k.n_cap == r->n_cap &&
-                          k.split == r->frame_split && k.state == (const void *)r->d_state;
-        if (!same) {
-            if (r->prep_exec) { cudaGraphExecDestroy(r->prep_exec); r->prep_exec = nullptr; }
-            if (!r->cap_stream) CU(cudaStreamCreateWithFlags(&r->cap_stream, cudaStreamNonBlocking));
-            CU(cudaStreamBeginCapture(r->cap_stream, cudaStreamCaptureModeThreadLocal));
-            st = enqueue_prepare_body(r, pc, r->cap_stream);
-            cudaGraph_t g = nullptr;
-            cudaError_t e = cudaStreamEndCapture(r->cap_stream, &g);
-            if (st != WS_OK) { if (g) cudaGraphDestroy(g); return st; }
-            if (e != cudaSuccess) return fail_cuda(e, "cudaStreamEndCapture");
-            e = cudaGraphInstantiate(&r->prep_exec, g, 0);
-            cudaGraphDestroy(g);
-            if (e != cudaSuccess) { r->prep_exec = nullptr; return fail_cuda(e, "cudaGraphInstantiate"); }
-            k.pc = pc; k.pc_gen = pc->generation; k.buf_gen = r->buf_generation; k.gaussians = pc->d_gaussians; k.scratch = r->d_scratch; k.n = pc->n; k.W = U.width; k.H = U.height;
-            k.pair_cap = r->pair_cap; k.n_cap = r->n_cap; k.split = r->frame_split; k.state = r->d_state;
-        }
-        CU(cudaGraphLaunch(r->prep_exec, stream));
-    } else {
-        st = enqueue_prepare_body(r, pc, stream);
-        if (st != WS_OK) return st;
+    *captured = false;
+    if (!r->use_graphs || r->timing) return body(stream);
+    if (!exec || !same) {
+        if (exec) { cudaGraphExecDestroy(exec); exec = nullptr; }
+        if (!r->cap_stream) CU(cudaStreamCreateWithFlags(&r->cap_stream, cudaStreamNonBlocking));
+        CU(cudaStreamBeginCapture(r->cap_stream, cudaStreamCaptureModeThreadLocal));
+        ws_status st = body(r->cap_stream);
+        cudaGraph_t g = nullptr;
+        cudaError_t e = cudaStreamEndCapture(r->cap_stream, &g);
+        if (st != WS_OK) { if (g) cudaGraphDestroy(g); return st; }
+        if (e != cudaSuccess) return fail_cuda(e, (std::string("cudaStreamEndCapture") + label).c_str());
+        e = cudaGraphInstantiate(&exec, g, 0);
+        cudaGraphDestroy(g);
+        if (e != cudaSuccess) { exec = nullptr; return fail_cuda(e, (std::string("cudaGraphInstantiate") + label).c_str()); }
+        *captured = true;
     }
+    CU(cudaGraphLaunch(exec, stream));
+    return WS_OK;
+}
+
+// Batches of views of one cloud (DESIGN.md "Batches of views").  The K views are stacked into one "tall" frame: tile
+// (x, y) of view v is tile (v * tiles_y + y) * tiles_x + x.  Stage 1 runs once over the cloud for all views (view-major
+// slots), stage 2 is the single-frame depth sort / binning / tile sort over the K * T tiles, and the compositor runs
+// with gridDim.z = K.  Within each tile the order is (depth key, slot) with slots in Gaussian-index order, exactly as
+// in a single frame, so every view is bit-identical to the same view rendered alone.
+//
+// ws_renderer_prepare is a single frame (K = 1, batch = false), ws_renderer_prepare_views a batch (batch = true, any
+// K): a batch of one view still runs the batch instantiation of stage 1.
+static ws_status prepare_frame(ws_renderer *r, ws_pointcloud *pc, const ws_splatting_args *args, uint32_t K, bool batch,
+                               cudaStream_t stream)
+{
+    for (uint32_t v = 0; v < K; v++) {
+        ws_status st = validate_frame(r, pc, &args[v]);
+        if (st != WS_OK) return st;
+        if (args[v].viewport[0] != args[0].viewport[0] || args[v].viewport[1] != args[0].viewport[1])
+            return fail(WS_ERR_INVALID_ARGUMENT, "the views of a batch must share the viewport");
+    }
+    if (!batch && r->shard.world > 1) return fail(WS_ERR_INVALID_ARGUMENT, "renderer is configured for sharding: use ws_renderer_shard_begin/exchange/finish");
+    if (batch && r->shard.world > 0) return fail(WS_ERR_INVALID_ARGUMENT, "batches of views are not supported on a sharded renderer");
+    const uint64_t kn = (uint64_t)K * pc->n;         // a cloud has < 2^30 points: only a batch can reach the limit
+    if (kn >= (1ull << 30)) return fail(WS_ERR_UNSUPPORTED, "num_views x num_points must be < 2^30 (30-bit look-back counts)");
+    CU(cudaSetDevice(r->ctx->device));
+    ws_status st = take_deferred_status(r);
+    if (st != WS_OK) return st;
+    const uint32_t W = args[0].viewport[0], H = args[0].viewport[1];
+    st = decide_split(r, kn, W, H, K);
+    if (st != WS_OK) return st;
+    st = begin_frame(r, pc, args, K, batch, (uint32_t)kn, stream, /*with_clears=*/false);   // capacities may (re)allocate
+    if (st != WS_OK) return st;
+
+    // clears + stage 1 + stage 2
+    auto body = [&](cudaStream_t q) -> ws_status {
+        CU(cudaMemsetAsync(r->d_scratch, 0, r->scratch_bytes, q));
+        CU(cudaMemsetAsync(r->d_ranges, 0xff, (size_t)r->tiles_cap * 8 * (r->frame_split ? 2 : 1), q));    // {begin, ~end} identities for atomicMin
+        if (r->timing) CU(cudaEventRecord(r->ev[EV_START], q));
+        CU(launch_preprocess(stage1_args(r, pc), r->compressed, batch, r->ctx->sm_count * 8, r->grid_pre[batch], q));
+        if (r->timing) CU(cudaEventRecord(r->ev[EV_PRE], q));
+        return enqueue_stage2(r, q);
+    };
+    // One CUDA graph per (cloud, viewport, views, capacities): 2 memsets + 14 kernels become one launch.  Every kernel
+    // reads its sizes (N, V, P) from device memory, so the graph is independent of the frame's content.
+    const PrepKey key = {pc, pc->generation, r->buf_generation, pc->d_gaussians, r->d_scratch, r->d_state,
+                         pc->n, K, W, H, r->pair_cap, r->n_cap, r->frame_split};
+    bool captured;
+    st = run_graph(r, r->prep_exec[batch], r->prep_key[batch] == key, &captured, batch ? " (batch of views)" : "", stream, body);
+    if (st != WS_OK) return st;
+    if (captured) r->prep_key[batch] = key;
     r->prepared = true;
     r->last_stream = stream;
     r->last_n = pc->n;
     return WS_OK;
 }
 
-// ------------------------------------------------------------------------------------
-// Batches of views of one cloud (DESIGN.md "Batches of views").  The K views are stacked into one "tall" frame: tile
-// (x, y) of view v is tile (v * tiles_y + y) * tiles_x + x.  Stage 1 runs once over the cloud for all views (view-major
-// slots), stage 2 is the single-frame depth sort / binning / tile sort over the K * T tiles, and the compositor runs
-// with gridDim.z = K.  Within each tile the order is (depth key, slot) with slots in Gaussian-index order, exactly as
-// in a single frame, so every view is bit-identical to the same view rendered alone.
-static ws_status enqueue_prepare_views_body(ws_renderer *r, ws_pointcloud *pc, cudaStream_t stream)
+extern "C" ws_status ws_renderer_prepare(ws_renderer *r, ws_pointcloud *pc, const ws_splatting_args *args, void *cuda_stream)
 {
-    CU(cudaMemsetAsync(r->d_scratch, 0, r->scratch_bytes, stream));
-    CU(cudaMemsetAsync(r->d_ranges, 0xff, (size_t)r->tiles_cap * 8 * (r->frame_split ? 2 : 1), stream));
-    if (r->timing) CU(cudaEventRecord(r->ev[EV_START], stream));
-    {
-        PreprocessArgs a;
-        a.gaussians = pc->d_gaussians; a.xyz = pc->d_xyz; a.sh_coefs = pc->d_sh; a.covars = pc->d_covars;
-        a.uniforms = r->d_uniforms + 1;                 // the K view-local blocks
-        a.splats = r->d_splats; a.depth_keys = r->d_keys[0]; a.slot_vals = r->d_vals[0]; a.rects = r->d_rects;
-        a.part_counts = r->d_scan_pre; a.part_bases = r->d_part_bases;
-        a.hist = r->d_hist_depth; a.counters = r->d_counters;
-        a.num_views = r->views; a.part_union = r->d_part_union; a.view_visible = r->d_view_visible;
-        CU(launch_preprocess_views(a, r->compressed, r->ctx->sm_count * 8, r->grid_pre_views, stream));
-    }
-    if (r->timing) CU(cudaEventRecord(r->ev[EV_PRE], stream));
-    return enqueue_stage2(r, stream);
+    return prepare_frame(r, pc, args, 1, false, (cudaStream_t)cuda_stream);
 }
 
 extern "C" ws_status ws_renderer_prepare_views(ws_renderer *r, ws_pointcloud *pc, const ws_splatting_args *args,
@@ -1265,71 +1287,7 @@ extern "C" ws_status ws_renderer_prepare_views(ws_renderer *r, ws_pointcloud *pc
 {
     if (!r || !pc || !args) return fail(WS_ERR_INVALID_ARGUMENT, "NULL argument");
     if (num_views == 0 || num_views > WS_MAX_VIEWS) return fail(WS_ERR_INVALID_ARGUMENT, "num_views must be in [1, WS_MAX_VIEWS]");
-    for (uint32_t v = 0; v < num_views; v++) {
-        ws_status st = validate_frame(r, pc, &args[v]);
-        if (st != WS_OK) return st;
-        if (args[v].viewport[0] != args[0].viewport[0] || args[v].viewport[1] != args[0].viewport[1])
-            return fail(WS_ERR_INVALID_ARGUMENT, "the views of a batch must share the viewport");
-    }
-    if (r->shard.world > 0) return fail(WS_ERR_INVALID_ARGUMENT, "batches of views are not supported on a sharded renderer");
-    const uint64_t kn = (uint64_t)num_views * pc->n;
-    if (kn >= (1ull << 30)) return fail(WS_ERR_UNSUPPORTED, "num_views x num_points must be < 2^30 (30-bit look-back counts)");
-    cudaStream_t stream = (cudaStream_t)cuda_stream;
-    CU(cudaSetDevice(r->ctx->device));
-    ws_status st = take_deferred_status(r);
-    if (st != WS_OK) return st;
-    const uint32_t K = num_views, W = args[0].viewport[0], H = args[0].viewport[1];
-    const uint32_t tx = (W + TILE - 1) / TILE, ty = (H + TILE - 1) / TILE;
-    const uint32_t tiles = tx * ty * K;              // < 2^23 for viewports up to 16384 and K <= 8
-    st = decide_split(r, kn, W, H, K);
-    if (st != WS_OK) return st;
-    r->prepared = false; r->rendered = false;
-    st = ensure_capacity(r, (uint32_t)kn, tiles, K);
-    if (st != WS_OK) return st;
-    uint32_t max_deg = 0;
-    for (uint32_t v = 0; v < K; v++) {
-        build_frame_uniforms(r, pc, &args[v], &r->h_views[1 + v]);
-        if (args[v].max_sh_deg > max_deg) max_deg = args[v].max_sh_deg;
-    }
-    FrameUniforms &T = r->h_views[0];                // stages 2-3: view 0's block with K * tiles_y tile rows
-    T = r->h_views[1];
-    T.tiles_y = ty * K;
-    T.rs.max_sh_deg = max_deg;                       // read only by ws_renderer_stats (SH bytes of the batch)
-    r->h_uniforms = T;
-    r->views = K; r->batch = true;
-    r->tile_passes = (tiles > 65536u) ? 3 : ((tiles > 256u) ? 2 : 1);
-    // one upload of the 1 + K blocks in front of the frame (pageable: staged before the call returns)
-    CU(cudaMemcpyAsync(r->d_uniforms, r->h_views, (1 + K) * sizeof(FrameUniforms), cudaMemcpyHostToDevice, stream));
-    if (r->use_graphs && !r->timing) {
-        auto &k = r->views_key;
-        const bool same = r->views_exec && k.pc == pc && k.pc_gen == pc->generation && k.buf_gen == r->buf_generation &&
-                          k.gaussians == pc->d_gaussians && k.scratch == r->d_scratch && k.n == pc->n && k.K == K &&
-                          k.W == W && k.H == H && k.pair_cap == r->pair_cap && k.n_cap == r->n_cap &&
-                          k.split == r->frame_split && k.state == (const void *)r->d_state;
-        if (!same) {
-            if (r->views_exec) { cudaGraphExecDestroy(r->views_exec); r->views_exec = nullptr; }
-            if (!r->cap_stream) CU(cudaStreamCreateWithFlags(&r->cap_stream, cudaStreamNonBlocking));
-            CU(cudaStreamBeginCapture(r->cap_stream, cudaStreamCaptureModeThreadLocal));
-            st = enqueue_prepare_views_body(r, pc, r->cap_stream);
-            cudaGraph_t g = nullptr;
-            cudaError_t e = cudaStreamEndCapture(r->cap_stream, &g);
-            if (st != WS_OK) { if (g) cudaGraphDestroy(g); return st; }
-            if (e != cudaSuccess) return fail_cuda(e, "cudaStreamEndCapture (batch of views)");
-            e = cudaGraphInstantiate(&r->views_exec, g, 0);
-            cudaGraphDestroy(g);
-            if (e != cudaSuccess) { r->views_exec = nullptr; return fail_cuda(e, "cudaGraphInstantiate (batch of views)"); }
-            k.pc = pc; k.pc_gen = pc->generation; k.buf_gen = r->buf_generation; k.gaussians = pc->d_gaussians; k.scratch = r->d_scratch;
-            k.n = pc->n; k.K = K; k.W = W; k.H = H; k.pair_cap = r->pair_cap; k.n_cap = r->n_cap; k.split = r->frame_split; k.state = r->d_state;
-        }
-        CU(cudaGraphLaunch(r->views_exec, stream));
-    } else {
-        st = enqueue_prepare_views_body(r, pc, stream);
-        if (st != WS_OK) return st;
-    }
-    r->prepared = true;
-    r->last_stream = stream;
-    r->last_n = pc->n;
-    return WS_OK;
+    return prepare_frame(r, pc, args, num_views, true, (cudaStream_t)cuda_stream);
 }
 
 // ------------------------------------------------------------------------------------
@@ -1485,18 +1443,15 @@ extern "C" ws_status ws_renderer_shard_begin(ws_renderer *r, ws_pointcloud *pc, 
     cudaStream_t stream = (cudaStream_t)cuda_stream;
     CU(cudaSetDevice(r->ctx->device));
     r->frame_split = false;
-    st = begin_frame(r, pc, args, s.recv_cap, stream);
+    st = begin_frame(r, pc, args, 1, false, s.recv_cap, stream);
     if (st != WS_OK) return st;
     if (r->timing) CU(cudaEventRecord(r->ev[EV_START], stream));
     {   // ---- stage 1 on the local shard, into the local staging arrays
-        PreprocessArgs a;
-        a.gaussians = pc->d_gaussians; a.xyz = pc->d_xyz; a.sh_coefs = pc->d_sh; a.covars = pc->d_covars;
-        a.uniforms = r->d_uniforms;
+        PreprocessArgs a = stage1_args(r, pc);
         a.splats = s.l_splats; a.depth_keys = s.l_keys; a.slot_vals = s.l_vals; a.rects = s.l_rects;
-        a.part_counts = r->d_scan_pre; a.part_bases = r->d_part_bases;
-        a.hist = s.hist_dummy; a.counters = r->d_counters;      // the consumer histograms the keys it RECEIVES
+        a.hist = s.hist_dummy;                                   // the consumer histograms the keys it RECEIVES
         CU(cudaMemsetAsync(s.hist_dummy, 0, 4 * 256 * 4, stream));
-        CU(launch_preprocess(a, r->compressed, r->ctx->sm_count * 8, r->grid_pre, stream));
+        CU(launch_preprocess(a, r->compressed, false, r->ctx->sm_count * 8, r->grid_pre[0], stream));
     }
     {   // ---- routing pass 1+2: how many local splats go to each band
         RouteArgs a; fill_route_args(r, a);
@@ -1570,7 +1525,7 @@ extern "C" ws_status ws_renderer_shard_frame_to_root(ws_renderer *r, ws_pointclo
     // rank's share of the cloud is large enough to pay for the extra launches (2 GPUs at cfg3: yes; 8 GPUs: no)
     st = decide_split(r, (uint64_t)s.recv_cap / s.world, s.width, s.height);
     if (st != WS_OK) return st;
-    st = begin_frame(r, pc, args, s.recv_cap, stream, /*with_clears=*/false);      // uniforms (an ordinary async copy in front of the frame)
+    st = begin_frame(r, pc, args, 1, false, s.recv_cap, stream, /*with_clears=*/false);      // uniforms (an ordinary async copy in front of the frame)
     if (st != WS_OK) return st;
     const uint32_t rows = s.band_y0[s.rank + 1] - s.band_y0[s.rank];
     if (rows == 0 || s.band_y0[s.rank] * TILE >= s.height) return fail(WS_ERR_UNSUPPORTED, "a rank without tile rows (more ranks than tile rows) is not supported");
@@ -1586,13 +1541,10 @@ extern "C" ws_status ws_renderer_shard_frame_to_root(ws_renderer *r, ws_pointclo
         CU(launch_epoch_advance(s.d_epoch, q));
         if (r->timing) CU(cudaEventRecord(r->ev[EV_START], q));
         {   // stage 1 on the local shard
-            PreprocessArgs a;
-            a.gaussians = pc->d_gaussians; a.xyz = pc->d_xyz; a.sh_coefs = pc->d_sh; a.covars = pc->d_covars;
-            a.uniforms = r->d_uniforms;
+            PreprocessArgs a = stage1_args(r, pc);
             a.splats = s.l_splats; a.depth_keys = s.l_keys; a.slot_vals = s.l_vals; a.rects = s.l_rects;
-            a.part_counts = r->d_scan_pre; a.part_bases = r->d_part_bases;
-            a.hist = s.hist_dummy; a.counters = r->d_counters;
-            CU(launch_preprocess(a, r->compressed, r->ctx->sm_count * 8, r->grid_pre, q));
+            a.hist = s.hist_dummy;
+            CU(launch_preprocess(a, r->compressed, false, r->ctx->sm_count * 8, r->grid_pre[0], q));
         }
         RouteArgs ra; fill_route_args(r, ra);
         for (uint32_t p = 0; p < s.world; p++) ra.peer_mail[p] = s.peer_mail[p];
@@ -1612,34 +1564,20 @@ extern "C" ws_status ws_renderer_shard_frame_to_root(ws_renderer *r, ws_pointclo
         return WS_OK;
     };
 
-    if (r->use_graphs && !r->timing) {
-        // One CUDA graph per frame-buffer parity: ~25 launches + 3 clears become one launch (host: ~200 -> ~60 us per
-        // frame and rank; device: no launch gaps between the latency-bound kernels of a 1/8 share of the frame).
-        auto &k = s.frame_key[par];
-        bool same = s.frame_exec[par] && k.pc_gen == pc->generation && k.buf_gen == r->buf_generation && k.root == root &&
-                    k.gated == s.gated && k.split == r->frame_split;
-        for (int i = 0; i < 9 && same; i++) same = k.bands[i] == s.band_y0[i];
-        for (int i = 0; i < 4 && same; i++) same = k.clear[i] == (clear ? (float)clear[i] : 0.f);
-        if (!same) {
-            if (s.frame_exec[par]) { cudaGraphExecDestroy(s.frame_exec[par]); s.frame_exec[par] = nullptr; }
-            if (!r->cap_stream) CU(cudaStreamCreateWithFlags(&r->cap_stream, cudaStreamNonBlocking));
-            CU(cudaStreamBeginCapture(r->cap_stream, cudaStreamCaptureModeThreadLocal));
-            st = body(r->cap_stream);
-            cudaGraph_t g = nullptr;
-            cudaError_t e = cudaStreamEndCapture(r->cap_stream, &g);
-            if (st != WS_OK) { if (g) cudaGraphDestroy(g); return st; }
-            if (e != cudaSuccess) return fail_cuda(e, "cudaStreamEndCapture (sharded frame)");
-            e = cudaGraphInstantiate(&s.frame_exec[par], g, 0);
-            cudaGraphDestroy(g);
-            if (e != cudaSuccess) { s.frame_exec[par] = nullptr; return fail_cuda(e, "cudaGraphInstantiate (sharded frame)"); }
-            k.pc_gen = pc->generation; k.buf_gen = r->buf_generation; k.root = root; k.gated = s.gated; k.split = r->frame_split;
-            for (int i = 0; i < 9; i++) k.bands[i] = s.band_y0[i];
-            for (int i = 0; i < 4; i++) k.clear[i] = clear ? (float)clear[i] : 0.f;
-        }
-        CU(cudaGraphLaunch(s.frame_exec[par], stream));
-    } else {
-        st = body(stream);
-        if (st != WS_OK) return st;
+    // One CUDA graph per frame-buffer parity: ~25 launches + 3 clears become one launch (host: ~200 -> ~60 us per
+    // frame and rank; device: no launch gaps between the latency-bound kernels of a 1/8 share of the frame).
+    auto &k = s.frame_key[par];
+    bool same = k.pc_gen == pc->generation && k.buf_gen == r->buf_generation && k.root == root && k.gated == s.gated &&
+                k.split == r->frame_split;
+    for (int i = 0; i < 9 && same; i++) same = k.bands[i] == s.band_y0[i];
+    for (int i = 0; i < 4 && same; i++) same = k.clear[i] == (clear ? (float)clear[i] : 0.f);
+    bool captured;
+    st = run_graph(r, s.frame_exec[par], same, &captured, " (sharded frame)", stream, body);
+    if (st != WS_OK) return st;
+    if (captured) {
+        k.pc_gen = pc->generation; k.buf_gen = r->buf_generation; k.root = root; k.gated = s.gated; k.split = r->frame_split;
+        for (int i = 0; i < 9; i++) k.bands[i] = s.band_y0[i];
+        for (int i = 0; i < 4; i++) k.clear[i] = clear ? (float)clear[i] : 0.f;
     }
     s.epoch += 1;
     st = enqueue_status_copy(r, stream);

@@ -14,6 +14,9 @@
 //    no inter-CTA dependency at all -- a single-pass chained scan was tried first (r01a/r01b in
 //    profiles/): its look-back serialised the prefetch pipeline.  The price is re-reading xyz:
 //    +12 B on top of 124 B per Gaussian;
+//  * each kernel is one template over <COMPRESSED, BATCH>.  BATCH = false is a single frame: one uniform block and
+//    K = 1 view at compile time.  BATCH = true is a batch of K <= MAX_VIEWS views of one cloud (DESIGN.md section 12):
+//    the records and SH are read once and every view is culled, projected and compacted from them, into view-major slots;
 //  * MAIN is software-pipelined: partitions are assigned round-robin, the 28-B (24-B) AoS
 //    records of partition k+1 and -- when at least half of it survives -- its 24-KB SH block
 //    are fetched by cp.async.bulk (TMA engine, UBLKCP) into shared-memory rings while
@@ -336,22 +339,24 @@ __device__ __forceinline__ bool cull_project(const FrameUniforms &U, float x, fl
 }
 
 // ---- (1) COUNT: survivors per partition + depth-key digit histograms -----------------------
-template <bool COMPRESSED>
+// BATCH: the K = a.num_views views are culled one after the other against the same positions; part_counts holds
+// K x nparts survivor counts (view-major) and part_union the Gaussians of each partition that survive in any view.
+template <bool COMPRESSED, bool BATCH>
 __global__ void __launch_bounds__(PP_THREADS)
 count_kernel(PreprocessArgs a)
 {
-    __shared__ FrameUniforms s_u;
+    __shared__ FrameUniforms s_u[BATCH ? MAX_VIEWS : 1u];
     __shared__ uint32_t s_hist[4 * 256];
     const unsigned tid = threadIdx.x;
+    const uint32_t K = BATCH ? a.num_views : 1u;
     {
         const uint32_t *src = reinterpret_cast<const uint32_t *>(a.uniforms);
-        uint32_t *dst = reinterpret_cast<uint32_t *>(&s_u);
-        for (unsigned i = tid; i < sizeof(FrameUniforms) / 4u; i += PP_THREADS) dst[i] = src[i];
+        uint32_t *dst = reinterpret_cast<uint32_t *>(s_u);
+        for (unsigned i = tid; i < K * (uint32_t)(sizeof(FrameUniforms) / 4u); i += PP_THREADS) dst[i] = src[i];
     }
     for (unsigned i = tid; i < 4u * 256u; i += PP_THREADS) s_hist[i] = 0u;
     __syncthreads();
-    const FrameUniforms &U = s_u;
-    const uint32_t n = U.num_points;
+    const uint32_t n = s_u[0].num_points;
     const uint32_t nparts = (n + PP_THREADS - 1u) / PP_THREADS;
     constexpr int NDIG = 4;
     // CNT_UNROLL consecutive partitions per trip: their 3 * CNT_UNROLL loads are issued before the first use, and the
@@ -367,27 +372,41 @@ count_kernel(PreprocessArgs a)
             const float *p = a.xyz + (size_t)idx * 3u;
             px[u] = __ldg(p); py[u] = __ldg(p + 1); pz[u] = __ldg(p + 2);
         }
-        bool keep[CNT_UNROLL];
-        uint32_t key[CNT_UNROLL];
+        bool any[CNT_UNROLL];                                              // BATCH: survives in at least one view
 #pragma unroll
-        for (uint32_t u = 0; u < CNT_UNROLL; u++) {
-            float cs[4], pp[4];
-            const bool valid = (part0 + u) * PP_THREADS + tid < n;
-            keep[u] = cull_project<COMPRESSED>(U, px[u], py[u], pz[u], cs, pp) && valid;
-            key[u] = depth_key<COMPRESSED>(U, pp[2]);
+        for (uint32_t u = 0; u < CNT_UNROLL; u++) any[u] = false;
+        for (uint32_t v = 0; v < K; v++) {
+            const FrameUniforms &U = s_u[v];
+            bool keep[CNT_UNROLL];
+            uint32_t key[CNT_UNROLL];
+#pragma unroll
+            for (uint32_t u = 0; u < CNT_UNROLL; u++) {
+                float cs[4], pp[4];
+                const bool valid = (part0 + u) * PP_THREADS + tid < n;
+                keep[u] = cull_project<COMPRESSED>(U, px[u], py[u], pz[u], cs, pp) && valid;
+                key[u] = depth_key<COMPRESSED>(U, pp[2]);
+                if (BATCH) any[u] = any[u] || keep[u];      // unguarded, it costs the single-view kernel 8 registers
+            }
+#pragma unroll
+            for (uint32_t u = 0; u < CNT_UNROLL; u++) {
+                const uint32_t cnt = (uint32_t)__syncthreads_count(keep[u] ? 1 : 0);
+                if (tid == 0 && part0 + u < nparts) a.part_counts[v * nparts + part0 + u] = cnt;
+            }
+            // shared atomics without return sustain ~120 G warp-ops/s on B200 whatever the spread
+            // (profiles/microbench/rank_primitives.cu); MATCH-aggregating them was 25x slower
+#pragma unroll
+            for (uint32_t u = 0; u < CNT_UNROLL; u++) {
+                if (keep[u]) {
+#pragma unroll
+                    for (int d = 0; d < NDIG; d++) atomicAdd(&s_hist[d * 256 + ((key[u] >> (8 * d)) & 255u)], 1u);
+                }
+            }
         }
+        if (BATCH) {
 #pragma unroll
-        for (uint32_t u = 0; u < CNT_UNROLL; u++) {
-            const uint32_t cnt = (uint32_t)__syncthreads_count(keep[u] ? 1 : 0);
-            if (tid == 0 && part0 + u < nparts) a.part_counts[part0 + u] = cnt;
-        }
-        // shared atomics without return sustain ~120 G warp-ops/s on B200 whatever the spread
-        // (profiles/microbench/rank_primitives.cu); MATCH-aggregating them was 25x slower
-#pragma unroll
-        for (uint32_t u = 0; u < CNT_UNROLL; u++) {
-            if (keep[u]) {
-#pragma unroll
-                for (int d = 0; d < NDIG; d++) atomicAdd(&s_hist[d * 256 + ((key[u] >> (8 * d)) & 255u)], 1u);
+            for (uint32_t u = 0; u < CNT_UNROLL; u++) {
+                const uint32_t cnt = (uint32_t)__syncthreads_count(any[u] ? 1 : 0);
+                if (tid == 0 && part0 + u < nparts) a.part_union[part0 + u] = cnt;
             }
         }
     }
@@ -399,14 +418,23 @@ count_kernel(PreprocessArgs a)
 }
 
 // ---- (2) SCAN: exclusive scan of the partition counts (one CTA) ------------------------------
+// BATCH: one scan over the K x nparts counts gives view-major slot bases, plus the per-view totals V_v
+template <bool BATCH>
 __global__ void __launch_bounds__(1024)
-scan_kernel(const uint32_t *__restrict__ counts, uint32_t *__restrict__ bases, const FrameUniforms *uniforms,
-            FrameCounters *counters)
+scan_kernel(PreprocessArgs a)
 {
-    const uint32_t n = uniforms->num_points;
-    const uint32_t nparts = (n + PP_THREADS - 1u) / PP_THREADS;
-    const uint32_t total = block_exclusive_scan_1024<uint32_t>(counts, bases, nparts);      // <= N < 2^32: 32-bit scan
-    if (threadIdx.x == 0) counters->num_visible = total;
+    const uint32_t K = BATCH ? a.num_views : 1u;
+    const uint32_t nparts = (a.uniforms->num_points + PP_THREADS - 1u) / PP_THREADS;
+    // a single frame has <= N < 2^32 survivors, a batch K * N < 2^30: a 32-bit scan
+    const uint32_t total = block_exclusive_scan_1024<uint32_t>(a.part_counts, a.part_bases, K * nparts);
+    // the scan ends with a barrier: every base written above is visible to the whole block
+    if (BATCH && threadIdx.x < K) {
+        const uint32_t v = threadIdx.x;
+        const uint32_t b0 = nparts ? a.part_bases[v * nparts] : 0u;
+        const uint32_t b1 = (nparts && v + 1u < K) ? a.part_bases[(v + 1u) * nparts] : total;
+        a.view_visible[v] = b1 - b0;
+    }
+    if (threadIdx.x == 0) a.counters->num_visible = total;
 }
 
 // ---- (3) MAIN ---------------------------------------------------------------------------------
@@ -430,27 +458,34 @@ struct PPSmem {
     static constexpr uint32_t off_lut = off_misc + 64u;                                        // compressed: 2 x 256 dequantised SH codes
     static constexpr uint32_t bytes = off_lut + (COMPRESSED ? 2u * 256u * 4u : 0u);
 };
+template <bool COMPRESSED, bool BATCH>
+using PPLayout = PPSmem<COMPRESSED, BATCH ? MAX_VIEWS : 1u>;
 
-template <bool COMPRESSED>
+// BATCH: each partition's records and SH are staged once and every view culls, projects and compacts from them in
+// turn, with the same cull_project / project_tail as a single frame (this file is built with -fmad=false), so each
+// view's halves, keys and rectangles are bit for bit those of the same view rendered alone.  View v's survivors take
+// the slots [B_v, B_v + V_v) in Gaussian-index order, and its rectangles are moved down to its rows of the "tall" frame.
+template <bool COMPRESSED, bool BATCH>
 __global__ void __launch_bounds__(PP_THREADS, 3)
 preprocess_kernel(PreprocessArgs a)
 {
-    using L = PPSmem<COMPRESSED>;
+    using L = PPLayout<COMPRESSED, BATCH>;
     constexpr uint32_t REC = L::REC, REC_WORDS = REC / 4u;
     extern __shared__ __align__(128) uint8_t smem[];
     uint32_t *s_splat = reinterpret_cast<uint32_t *>(smem + L::off_splat);
     uint32_t *s_key = reinterpret_cast<uint32_t *>(smem + L::off_key);
     uint2 *s_rect = reinterpret_cast<uint2 *>(smem + L::off_rect);
-    FrameUniforms &s_u = *reinterpret_cast<FrameUniforms *>(smem + L::off_u);
+    const FrameUniforms *s_u = reinterpret_cast<const FrameUniforms *>(smem + L::off_u);
     uint64_t *s_rbar = reinterpret_cast<uint64_t *>(smem + L::off_bar);
     uint64_t *s_sbar = s_rbar + PP_STAGES;
     uint32_t *s_warp_cnt = reinterpret_cast<uint32_t *>(smem + L::off_misc);      // [8]
 
     const unsigned tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
+    const uint32_t K = BATCH ? a.num_views : 1u;
     {   // uniforms -> smem
         const uint32_t *src = reinterpret_cast<const uint32_t *>(a.uniforms);
-        uint32_t *dst = reinterpret_cast<uint32_t *>(&s_u);
-        for (unsigned i = tid; i < sizeof(FrameUniforms) / 4u; i += PP_THREADS) dst[i] = src[i];
+        uint32_t *dst = reinterpret_cast<uint32_t *>(smem + L::off_u);
+        for (unsigned i = tid; i < K * (uint32_t)(sizeof(FrameUniforms) / 4u); i += PP_THREADS) dst[i] = src[i];
     }
     if (tid == 0) {
         for (int i = 0; i < 2 * PP_STAGES; i++) mbar_init(&s_rbar[i], 1);
@@ -458,20 +493,23 @@ preprocess_kernel(PreprocessArgs a)
     }
     float *s_lut = reinterpret_cast<float *>(smem + L::off_lut);
     if (COMPRESSED) {
-        const FrameUniforms *gu = a.uniforms;                    // s_u is not visible yet: read the two quantisers from global
+        // s_u is not visible yet: read the two quantisers from global (they belong to the cloud: the same in every view)
+        const FrameUniforms *gu = a.uniforms;
         const Quant qd = gu->quant.color_dc, qr = gu->quant.color_rest;
         s_lut[tid] = ShQuant::dq((int8_t)tid, qd);               // index = the byte's bit pattern
         s_lut[256 + tid] = ShQuant::dq((int8_t)tid, qr);
     }
     __syncthreads();
-    const FrameUniforms &U = s_u;
-    const uint32_t n = U.num_points;
+    const uint32_t n = s_u[0].num_points;
     const uint32_t nparts = (n + PP_THREADS - 1u) / PP_THREADS;
-    const bool sh_bulk_ok = !COMPRESSED && U.rs.max_sh_deg >= 2u;
+    uint32_t max_deg = s_u[0].rs.max_sh_deg;                     // SH is fetched once, for the highest degree of the batch
+    for (uint32_t v = 1; v < K; v++) max_deg = s_u[v].rs.max_sh_deg > max_deg ? s_u[v].rs.max_sh_deg : max_deg;
+    const bool sh_bulk_ok = !COMPRESSED && max_deg >= 2u;
+    const uint32_t *survivors = BATCH ? a.part_union : a.part_counts;     // a batch: survivors in at least one view
 
     // iteration k of this CTA handles partition blockIdx.x + k * gridDim.x
     auto part_of = [&](uint32_t k) -> uint32_t { return blockIdx.x + k * gridDim.x; };
-    auto uses_bulk_sh = [&](uint32_t part) -> bool { return sh_bulk_ok && __ldg(a.part_counts + part) >= PP_SH_BULK_MIN; };
+    auto uses_bulk_sh = [&](uint32_t part) -> bool { return sh_bulk_ok && __ldg(survivors + part) >= PP_SH_BULK_MIN; };
     auto issue = [&](uint32_t k) {                    // thread 0 only: fetch everything partition k needs
         const uint32_t part = part_of(k);
         if (part >= nparts) return;
@@ -493,249 +531,6 @@ preprocess_kernel(PreprocessArgs a)
         if (part >= nparts) break;
         const uint32_t s = k % PP_STAGES;
         if (tid == 0) issue(k + 1u);                  // slot (k+1)%2 was last read in iteration k-1 (trailing barrier)
-
-        const bool bulk = uses_bulk_sh(part);
-        mbar_wait(&s_rbar[s], (rpar >> s) & 1u); rpar ^= 1u << s;
-        if (bulk) { mbar_wait(&s_sbar[s], (spar >> s) & 1u); spar ^= 1u << s; }
-
-        const uint32_t *rec = reinterpret_cast<const uint32_t *>(smem + L::off_rec + s * L::REC_BYTES) + tid * REC_WORDS;
-        const uint32_t idx = part * PP_THREADS + tid;
-        bool vis = false;
-        Stage1 o;
-        o.key = 0u; o.rect_xy = 0u; o.rect_wh = 0u;
-        o.splat[0] = o.splat[1] = o.splat[2] = o.splat[3] = o.splat[4] = 0u;
-        if (idx < n) {
-            const float x = __uint_as_float(rec[0]), y = __uint_as_float(rec[1]), z = __uint_as_float(rec[2]);
-            float cs[4], pp[4];
-            if (cull_project<COMPRESSED>(U, x, y, z, cs, pp)) {
-                vis = true;
-                if (!COMPRESSED) {
-                    const float opacity = half_lo(rec[3]);
-                    const float cov6[6] = {half_lo(rec[4]), half_hi(rec[4]), half_lo(rec[5]),
-                                           half_hi(rec[5]), half_lo(rec[6]), half_hi(rec[6])};
-                    ShRaw sh;
-                    const uint32_t deg = U.rs.max_sh_deg;
-                    if (bulk) {
-                        const uint4 *sp = reinterpret_cast<const uint4 *>(smem + L::off_sh + s * PP_SH_BYTES + tid * 96u);
-#pragma unroll
-                        for (int q = 0; q < 6; q++) {
-                            const uint4 v = sp[q];
-                            sh.w[4 * q] = v.x; sh.w[4 * q + 1] = v.y; sh.w[4 * q + 2] = v.z; sh.w[4 * q + 3] = v.w;
-                        }
-                    } else {
-                        const uint8_t *sp = a.sh_coefs + (size_t)idx * 96u;
-                        ldg256(sp, sh.w);
-                        if (deg > 1u) ldg256(sp + 32, sh.w + 8); else {
-#pragma unroll
-                            for (int i = 8; i < 16; i++) sh.w[i] = 0u;
-                        }
-                        if (deg > 2u) ldg256(sp + 64, sh.w + 16); else {
-#pragma unroll
-                            for (int i = 16; i < 24; i++) sh.w[i] = 0u;
-                        }
-                    }
-                    project_tail<false>(U, x, y, z, cs[0], cs[1], cs[2], pp[0], pp[1], pp[2], pp[3], cov6, opacity, sh, o);
-                } else {
-                    const uint32_t os = rec[3];
-                    const int8_t q_op = (int8_t)(os & 0xffu), q_sf = (int8_t)((os >> 8) & 0xffu);
-                    const uint32_t geo_idx = rec[4], sh_idx = rec[5];
-                    const float opacity = ((float)q_op - (float)U.quant.opacity.zero_point) * U.quant.opacity.scale;
-                    const float sfac = expf(((float)q_sf - (float)U.quant.scaling_factor.zero_point) * U.quant.scaling_factor.scale);
-                    const float s2 = sfac * sfac;
-                    const uint32_t *cw = reinterpret_cast<const uint32_t *>(a.covars + (size_t)geo_idx * 12u);
-                    const uint32_t w0 = __ldg(cw), w1 = __ldg(cw + 1), w2 = __ldg(cw + 2);
-                    const float cov6[6] = {half_lo(w0) * s2, half_hi(w0) * s2, half_lo(w1) * s2,
-                                           half_hi(w1) * s2, half_lo(w2) * s2, half_hi(w2) * s2};
-                    const uint32_t ncoef = (U.file_sh_deg + 1u) * (U.file_sh_deg + 1u);
-                    ShQuant sh;
-                    sh.load(a.sh_coefs, sh_idx, ncoef);
-                    sh.lut = s_lut;
-                    project_tail<true>(U, x, y, z, cs[0], cs[1], cs[2], pp[0], pp[1], pp[2], pp[3], cov6, opacity, sh, o);
-                }
-            }
-        }
-
-        // ---- deterministic compaction: slot = scanned partition base + rank inside the partition
-        const unsigned bal = __ballot_sync(0xffffffffu, vis);
-        if (lane == 0) s_warp_cnt[warp] = __popc(bal);
-        __syncthreads();
-        uint32_t warp_off = 0, total = 0;
-#pragma unroll
-        for (int w = 0; w < PP_WARPS; w++) {
-            uint32_t c = s_warp_cnt[w];
-            if (w < (int)warp) warp_off += c;
-            total += c;
-        }
-        const uint32_t local = warp_off + __popc(bal & lanemask_lt());
-        if (vis) {
-#pragma unroll
-            for (int q = 0; q < 5; q++) s_splat[local * 5u + q] = o.splat[q];
-            s_key[local] = o.key;
-            s_rect[local] = make_uint2(o.rect_xy, o.rect_wh);
-        }
-        __syncthreads();
-        const uint32_t base = __ldg(a.part_bases + part);
-        // ---- coalesced output streams ----
-        for (uint32_t i = tid; i < total * 5u; i += PP_THREADS) a.splats[(size_t)base * 5u + i] = s_splat[i];
-        if (tid < total) {
-            a.depth_keys[base + tid] = s_key[tid];
-            a.slot_vals[base + tid] = base + tid;           // payload = slot, preprocess.wgsl:274
-            a.rects[base + tid] = s_rect[tid];
-        }
-        __syncthreads();
-    }
-}
-
-// ---- batches of views of one cloud (ws_renderer_prepare_views) --------------------------------
-// The same three launches over K <= MAX_VIEWS views.  Each Gaussian's position, record and SH are read once per batch and
-// culled / projected against every view with the single-view cull_project / project_tail (this file is built with
-// -fmad=false), so each view's halves, keys and rectangles are bit for bit those of the single-view kernels.
-// part_counts holds K x nparts survivor counts, view-major: their scan gives view v's survivors the slots
-// [B_v, B_v + V_v) in Gaussian-index order.  `a.uniforms` points at the K view-local uniform blocks.
-template <bool COMPRESSED>
-__global__ void __launch_bounds__(PP_THREADS)
-count_views_kernel(PreprocessArgs a)
-{
-    __shared__ FrameUniforms s_u[MAX_VIEWS];
-    __shared__ uint32_t s_hist[4 * 256];
-    const unsigned tid = threadIdx.x;
-    const uint32_t K = a.num_views;
-    {
-        const uint32_t *src = reinterpret_cast<const uint32_t *>(a.uniforms);
-        uint32_t *dst = reinterpret_cast<uint32_t *>(s_u);
-        for (unsigned i = tid; i < K * (uint32_t)(sizeof(FrameUniforms) / 4u); i += PP_THREADS) dst[i] = src[i];
-    }
-    for (unsigned i = tid; i < 4u * 256u; i += PP_THREADS) s_hist[i] = 0u;
-    __syncthreads();
-    const uint32_t n = s_u[0].num_points;
-    const uint32_t nparts = (n + PP_THREADS - 1u) / PP_THREADS;
-    constexpr uint32_t CNT_UNROLL = 4;
-    for (uint32_t part0 = blockIdx.x * CNT_UNROLL; part0 < nparts; part0 += gridDim.x * CNT_UNROLL) {
-        float px[CNT_UNROLL], py[CNT_UNROLL], pz[CNT_UNROLL];
-#pragma unroll
-        for (uint32_t u = 0; u < CNT_UNROLL; u++) {
-            uint32_t idx = (part0 + u) * PP_THREADS + tid;
-            idx = idx < n ? idx : n - 1u;
-            const float *p = a.xyz + (size_t)idx * 3u;
-            px[u] = __ldg(p); py[u] = __ldg(p + 1); pz[u] = __ldg(p + 2);
-        }
-        bool any[CNT_UNROLL];
-#pragma unroll
-        for (uint32_t u = 0; u < CNT_UNROLL; u++) any[u] = false;
-        for (uint32_t v = 0; v < K; v++) {
-            const FrameUniforms &U = s_u[v];
-            bool keep[CNT_UNROLL];
-#pragma unroll
-            for (uint32_t u = 0; u < CNT_UNROLL; u++) {
-                float cs[4], pp[4];
-                const bool valid = (part0 + u) * PP_THREADS + tid < n;
-                keep[u] = cull_project<COMPRESSED>(U, px[u], py[u], pz[u], cs, pp) && valid;
-                any[u] = any[u] || keep[u];
-                if (keep[u]) {
-                    const uint32_t key = depth_key<COMPRESSED>(U, pp[2]);
-#pragma unroll
-                    for (int d = 0; d < 4; d++) atomicAdd(&s_hist[d * 256 + ((key >> (8 * d)) & 255u)], 1u);
-                }
-            }
-#pragma unroll
-            for (uint32_t u = 0; u < CNT_UNROLL; u++) {
-                const uint32_t cnt = (uint32_t)__syncthreads_count(keep[u] ? 1 : 0);
-                if (tid == 0 && part0 + u < nparts) a.part_counts[v * nparts + part0 + u] = cnt;
-            }
-        }
-#pragma unroll
-        for (uint32_t u = 0; u < CNT_UNROLL; u++) {          // Gaussians that survive in at least one view
-            const uint32_t cnt = (uint32_t)__syncthreads_count(any[u] ? 1 : 0);
-            if (tid == 0 && part0 + u < nparts) a.part_union[part0 + u] = cnt;
-        }
-    }
-    __syncthreads();
-    for (unsigned i = tid; i < 4u * 256u; i += PP_THREADS) {
-        const uint32_t c = s_hist[i];
-        if (c) atomicAdd(a.hist + i, c);
-    }
-}
-
-// one scan over the K x nparts counts (view-major slot bases) + the per-view totals V_v
-__global__ void __launch_bounds__(1024)
-scan_views_kernel(PreprocessArgs a)
-{
-    const uint32_t K = a.num_views;
-    const uint32_t nparts = (a.uniforms->num_points + PP_THREADS - 1u) / PP_THREADS;
-    const uint32_t total = block_exclusive_scan_1024<uint32_t>(a.part_counts, a.part_bases, K * nparts);   // K * N < 2^30
-    // the scan ends with a barrier: every base written above is visible to the whole block
-    if (threadIdx.x < K) {
-        const uint32_t v = threadIdx.x;
-        const uint32_t b0 = nparts ? a.part_bases[v * nparts] : 0u;
-        const uint32_t b1 = (nparts && v + 1u < K) ? a.part_bases[(v + 1u) * nparts] : total;
-        a.view_visible[v] = b1 - b0;
-    }
-    if (threadIdx.x == 0) a.counters->num_visible = total;
-}
-
-template <bool COMPRESSED>
-__global__ void __launch_bounds__(PP_THREADS, 3)
-preprocess_views_kernel(PreprocessArgs a)
-{
-    using L = PPSmem<COMPRESSED, MAX_VIEWS>;
-    constexpr uint32_t REC = L::REC, REC_WORDS = REC / 4u;
-    extern __shared__ __align__(128) uint8_t smem[];
-    uint32_t *s_splat = reinterpret_cast<uint32_t *>(smem + L::off_splat);
-    uint32_t *s_key = reinterpret_cast<uint32_t *>(smem + L::off_key);
-    uint2 *s_rect = reinterpret_cast<uint2 *>(smem + L::off_rect);
-    const FrameUniforms *s_u = reinterpret_cast<const FrameUniforms *>(smem + L::off_u);
-    uint64_t *s_rbar = reinterpret_cast<uint64_t *>(smem + L::off_bar);
-    uint64_t *s_sbar = s_rbar + PP_STAGES;
-    uint32_t *s_warp_cnt = reinterpret_cast<uint32_t *>(smem + L::off_misc);      // [8]
-
-    const unsigned tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
-    const uint32_t K = a.num_views;
-    {
-        const uint32_t *src = reinterpret_cast<const uint32_t *>(a.uniforms);
-        uint32_t *dst = reinterpret_cast<uint32_t *>(smem + L::off_u);
-        for (unsigned i = tid; i < K * (uint32_t)(sizeof(FrameUniforms) / 4u); i += PP_THREADS) dst[i] = src[i];
-    }
-    if (tid == 0) {
-        for (int i = 0; i < 2 * PP_STAGES; i++) mbar_init(&s_rbar[i], 1);
-        fence_mbar_init();
-    }
-    float *s_lut = reinterpret_cast<float *>(smem + L::off_lut);
-    if (COMPRESSED) {                                            // the quantisers belong to the cloud: the same in every view
-        const Quant qd = a.uniforms->quant.color_dc, qr = a.uniforms->quant.color_rest;
-        s_lut[tid] = ShQuant::dq((int8_t)tid, qd);
-        s_lut[256 + tid] = ShQuant::dq((int8_t)tid, qr);
-    }
-    __syncthreads();
-    const uint32_t n = s_u[0].num_points;
-    const uint32_t nparts = (n + PP_THREADS - 1u) / PP_THREADS;
-    uint32_t max_deg = 0;                                        // SH is fetched once, for the highest degree of the batch
-    for (uint32_t v = 0; v < K; v++) max_deg = s_u[v].rs.max_sh_deg > max_deg ? s_u[v].rs.max_sh_deg : max_deg;
-    const bool sh_bulk_ok = !COMPRESSED && max_deg >= 2u;
-
-    auto part_of = [&](uint32_t k) -> uint32_t { return blockIdx.x + k * gridDim.x; };
-    // bulk-stage the SH block when at least half of the partition survives in some view
-    auto uses_bulk_sh = [&](uint32_t part) -> bool { return sh_bulk_ok && __ldg(a.part_union + part) >= PP_SH_BULK_MIN; };
-    auto issue = [&](uint32_t k) {
-        const uint32_t part = part_of(k);
-        if (part >= nparts) return;
-        const uint32_t s = k % PP_STAGES;
-        fence_proxy_async();
-        mbar_arrive_expect_tx(&s_rbar[s], L::REC_BYTES);
-        bulk_g2s(smem + L::off_rec + s * L::REC_BYTES, a.gaussians + (size_t)part * L::REC_BYTES, L::REC_BYTES, &s_rbar[s]);
-        if (uses_bulk_sh(part)) {
-            mbar_arrive_expect_tx(&s_sbar[s], PP_SH_BYTES);
-            bulk_g2s(smem + L::off_sh + s * PP_SH_BYTES, a.sh_coefs + (size_t)part * PP_SH_BYTES, PP_SH_BYTES, &s_sbar[s]);
-        }
-    };
-
-    if (tid == 0) issue(0);
-    uint32_t rpar = 0, spar = 0;
-
-    for (uint32_t k = 0;; k++) {
-        const uint32_t part = part_of(k);
-        if (part >= nparts) break;
-        const uint32_t s = k % PP_STAGES;
-        if (tid == 0) issue(k + 1u);
 
         const bool bulk = uses_bulk_sh(part);
         mbar_wait(&s_rbar[s], (rpar >> s) & 1u); rpar ^= 1u << s;
@@ -801,10 +596,10 @@ preprocess_views_kernel(PreprocessArgs a)
                     }
                 }
                 project_tail<COMPRESSED>(U, x, y, z, cs[0], cs[1], cs[2], pp[0], pp[1], pp[2], pp[3], cov6, opacity, sh, o);
-                if (o.rect_wh) o.rect_xy += (v * U.tiles_y) << 16;      // view v's tile rows in the "tall" frame
+                if (BATCH && o.rect_wh) o.rect_xy += (v * U.tiles_y) << 16;      // view v's tile rows in the "tall" frame
             }
 
-            // ---- deterministic compaction of view v: slot = scanned (view, partition) base + rank inside the partition
+            // ---- deterministic compaction: slot = scanned (view, partition) base + rank inside the partition
             const unsigned bal = __ballot_sync(0xffffffffu, vis);
             if (lane == 0) s_warp_cnt[warp] = __popc(bal);
             __syncthreads();
@@ -824,10 +619,11 @@ preprocess_views_kernel(PreprocessArgs a)
             }
             __syncthreads();
             const uint32_t base = __ldg(a.part_bases + v * nparts + part);
+            // ---- coalesced output streams ----
             for (uint32_t i = tid; i < total * 5u; i += PP_THREADS) a.splats[(size_t)base * 5u + i] = s_splat[i];
             if (tid < total) {
                 a.depth_keys[base + tid] = s_key[tid];
-                a.slot_vals[base + tid] = base + tid;
+                a.slot_vals[base + tid] = base + tid;           // payload = slot, preprocess.wgsl:274
                 a.rects[base + tid] = s_rect[tid];
             }
             __syncthreads();
@@ -839,7 +635,7 @@ preprocess_views_kernel(PreprocessArgs a)
 
 // The opt-in above 48 KB of dynamic shared memory is a per-device attribute: the C ABI allows several ws_context on
 // different devices in one process, so it is tracked per device (and per layout).
-template <bool C>
+template <bool C, bool B>
 static cudaError_t pp_prepare()
 {
     static bool done[64] = {};
@@ -847,73 +643,42 @@ static cudaError_t pp_prepare()
     cudaError_t e = cudaGetDevice(&dev);
     if (e != cudaSuccess) return e;
     if (dev >= 0 && dev < 64 && done[dev]) return cudaSuccess;
-    e = cudaFuncSetAttribute(preprocess_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PPSmem<C>::bytes);
+    e = cudaFuncSetAttribute(preprocess_kernel<C, B>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PPLayout<C, B>::bytes);
     if (e == cudaSuccess && dev >= 0 && dev < 64) done[dev] = true;
     return e;
 }
 
-template <bool C>
-static cudaError_t pp_views_prepare()
+template <bool C, bool B>
+static cudaError_t pp_launch(const PreprocessArgs &a, int grid_count, int grid_main, cudaStream_t stream)
 {
-    static bool done[64] = {};
-    int dev = 0;
-    cudaError_t e = cudaGetDevice(&dev);
+    cudaError_t e = pp_prepare<C, B>();
     if (e != cudaSuccess) return e;
-    if (dev >= 0 && dev < 64 && done[dev]) return cudaSuccess;
-    e = cudaFuncSetAttribute(preprocess_views_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PPSmem<C, MAX_VIEWS>::bytes);
-    if (e == cudaSuccess && dev >= 0 && dev < 64) done[dev] = true;
-    return e;
-}
-
-cudaError_t launch_preprocess_views(const PreprocessArgs &a, bool compressed, int grid_count, int grid_main, cudaStream_t stream)
-{
-    if (a.num_views < 1 || a.num_views > MAX_VIEWS) return cudaErrorInvalidValue;
-    cudaError_t e = compressed ? pp_views_prepare<true>() : pp_views_prepare<false>();
-    if (e != cudaSuccess) return e;
-    if (compressed) count_views_kernel<true><<<grid_count, PP_THREADS, 0, stream>>>(a);
-    else count_views_kernel<false><<<grid_count, PP_THREADS, 0, stream>>>(a);
-    scan_views_kernel<<<1, 1024, 0, stream>>>(a);
-    if (compressed) preprocess_views_kernel<true><<<grid_main, PP_THREADS, PPSmem<true, MAX_VIEWS>::bytes, stream>>>(a);
-    else preprocess_views_kernel<false><<<grid_main, PP_THREADS, PPSmem<false, MAX_VIEWS>::bytes, stream>>>(a);
+    count_kernel<C, B><<<grid_count, PP_THREADS, 0, stream>>>(a);
+    scan_kernel<B><<<1, 1024, 0, stream>>>(a);
+    preprocess_kernel<C, B><<<grid_main, PP_THREADS, PPLayout<C, B>::bytes, stream>>>(a);
     return cudaGetLastError();
 }
 
-int preprocess_views_blocks_per_sm(bool compressed)
+template <bool C, bool B>
+static int pp_blocks_per_sm()
 {
     int nb = 0;
-    if (compressed) {
-        if (pp_views_prepare<true>() != cudaSuccess) return 1;
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, preprocess_views_kernel<true>, PP_THREADS, PPSmem<true, MAX_VIEWS>::bytes);
-    } else {
-        if (pp_views_prepare<false>() != cudaSuccess) return 1;
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, preprocess_views_kernel<false>, PP_THREADS, PPSmem<false, MAX_VIEWS>::bytes);
-    }
+    if (pp_prepare<C, B>() != cudaSuccess) return 1;
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, preprocess_kernel<C, B>, PP_THREADS, PPLayout<C, B>::bytes);
     return nb > 0 ? nb : 1;
 }
 
-cudaError_t launch_preprocess(const PreprocessArgs &a, bool compressed, int grid_count, int grid_main, cudaStream_t stream)
+cudaError_t launch_preprocess(const PreprocessArgs &a, bool compressed, bool batch, int grid_count, int grid_main, cudaStream_t stream)
 {
-    cudaError_t e = compressed ? pp_prepare<true>() : pp_prepare<false>();
-    if (e != cudaSuccess) return e;
-    if (compressed) count_kernel<true><<<grid_count, PP_THREADS, 0, stream>>>(a);
-    else count_kernel<false><<<grid_count, PP_THREADS, 0, stream>>>(a);
-    scan_kernel<<<1, 1024, 0, stream>>>(a.part_counts, a.part_bases, a.uniforms, a.counters);
-    if (compressed) preprocess_kernel<true><<<grid_main, PP_THREADS, PPSmem<true>::bytes, stream>>>(a);
-    else preprocess_kernel<false><<<grid_main, PP_THREADS, PPSmem<false>::bytes, stream>>>(a);
-    return cudaGetLastError();
+    if (batch && (a.num_views < 1 || a.num_views > MAX_VIEWS)) return cudaErrorInvalidValue;
+    if (compressed) return batch ? pp_launch<true, true>(a, grid_count, grid_main, stream) : pp_launch<true, false>(a, grid_count, grid_main, stream);
+    return batch ? pp_launch<false, true>(a, grid_count, grid_main, stream) : pp_launch<false, false>(a, grid_count, grid_main, stream);
 }
 
-int preprocess_blocks_per_sm(bool compressed)
+int preprocess_blocks_per_sm(bool compressed, bool batch)
 {
-    int nb = 0;
-    if (compressed) {
-        if (pp_prepare<true>() != cudaSuccess) return 1;
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, preprocess_kernel<true>, PP_THREADS, PPSmem<true>::bytes);
-    } else {
-        if (pp_prepare<false>() != cudaSuccess) return 1;
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, preprocess_kernel<false>, PP_THREADS, PPSmem<false>::bytes);
-    }
-    return nb > 0 ? nb : 1;
+    if (compressed) return batch ? pp_blocks_per_sm<true, true>() : pp_blocks_per_sm<true, false>();
+    return batch ? pp_blocks_per_sm<false, true>() : pp_blocks_per_sm<false, false>();
 }
 
 }  // namespace ws

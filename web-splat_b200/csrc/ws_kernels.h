@@ -20,21 +20,19 @@ struct PreprocessArgs {
     uint32_t *depth_keys;         // out: V
     uint32_t *slot_vals;          // out: V (iota payload)
     uint2 *rects;                 // out: V x {x0 | y0<<16, w | h<<16}
-    uint32_t *part_counts;        // ceil(N/256): survivors per partition (count kernel)
-    uint32_t *part_bases;         // ceil(N/256): exclusive scan of part_counts (scan kernel)
+    uint32_t *part_counts;        // ceil(N/256) (batch: num_views x ceil(N/256), view-major): survivors per partition (count kernel)
+    uint32_t *part_bases;         // as part_counts: its exclusive scan (scan kernel)
     uint32_t *hist;               // 4 x 256 depth-key digit histograms (zeroed per frame)
     FrameCounters *counters;
-    // batches of views only (launch_preprocess_views): `uniforms` then points at num_views view-local blocks,
-    // part_counts / part_bases hold num_views x ceil(N/256) entries (view-major)
+    // read by the batch kernels only (batch = true): `uniforms` then points at num_views view-local blocks
     uint32_t num_views;
     uint32_t *part_union;         // ceil(N/256): Gaussians of the partition that survive in at least one view
     uint32_t *view_visible;       // out: num_views per-view survivor counts V_v
 };
-cudaError_t launch_preprocess(const PreprocessArgs &a, bool compressed, int grid_count, int grid_main, cudaStream_t stream);
-int preprocess_blocks_per_sm(bool compressed);
 constexpr uint32_t MAX_VIEWS = 8;  // views per batch (WS_MAX_VIEWS)
-cudaError_t launch_preprocess_views(const PreprocessArgs &a, bool compressed, int grid_count, int grid_main, cudaStream_t stream);
-int preprocess_views_blocks_per_sm(bool compressed);
+// batch: the kernels of a batch of 1..MAX_VIEWS views of one cloud; otherwise a single frame, which reads one uniform block
+cudaError_t launch_preprocess(const PreprocessArgs &a, bool compressed, bool batch, int grid_count, int grid_main, cudaStream_t stream);
+int preprocess_blocks_per_sm(bool compressed, bool batch);
 
 // ---- onesweep radix sort of (u32 key, u32 value) pairs ---------------------------
 constexpr int SORT_THREADS = 256;
